@@ -19,6 +19,11 @@ Every timed region performs at least one averaging round (with ``--meta-steps`` 
 (``--meta-epochs``^2 passes over ``--val-texts`` sequences @ ``--val-seq``, run by all ranks) + averaging + base broadcast.
 Data: synthetic tokens; weights: random init.  ``--impl reference`` = the unmodified upstream miner, ``--impl torch-bf16`` = HF
 GPT-2 under bf16 autocast + SDPA + fused AdamW + NCCL round (the strongest stock-library baseline).
+
+``--dump-outputs DIR`` writes what the ``value`` region computed, as float32 ``.npy`` files (rank 0): ``loss`` (the mean loss
+of its last step), ``theta_sample`` (a fixed, seeded sample of the fp32 weights the next step starts from) and ``mixer_w``
+(the mixing weights [miners, tensors] of its last round).  Inputs and initial weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -60,6 +65,8 @@ def parse_args(argv=None):
     ap.add_argument("--dropout", type=float, default=None, help="train-mode dropout; default = the model preset (GPT-2: 0.1, as in the reference)")
     ap.add_argument("--fp8-forward", action="store_true", help="e4m3 forward GEMMs with delayed scaling (config 4)")
     ap.add_argument("--fp8-backward", action="store_true", help="with --fp8-forward: fp8 dgrad GEMMs (e5m2 gradients x transposed e4m3 weights)")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write the loss, weights (seeded sample) and mixing weights of the timed steps to DIR/<name>.npy")
     return ap.parse_args(argv)
 
 
@@ -72,6 +79,32 @@ def shared_config(model_desc: str, B: int, T: int, world: int) -> dict:
 
 
 GPT2_SMALL_DESC = "gpt2-small + [PAD] (124440576 params, vocab 50258)"
+DUMP_THETA_SAMPLE = 1 << 22  # fp32 weights kept by --dump-outputs: 16 MB, whatever the model size
+
+
+def capture_outputs(trainer, coord) -> dict:
+    """Host copies of what a caller of the timed steps holds after the last one: that step's loss, the weights the next
+    step starts from (a fixed, seeded sample) and the mixing weights.  Reads only: the trainer's state is left as it is."""
+    import torch
+
+    coord.sync_base()  # a base pushed by the peers must have landed before it is read
+    theta = trainer.base if trainer.master_stale else trainer.master  # right after a round theta lives in theta_base
+    n = theta.numel()
+    if n <= DUMP_THETA_SAMPLE:
+        idx = torch.arange(n)
+    else:
+        idx = torch.randint(n, (DUMP_THETA_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    out = {"loss": trainer.engine.loss.reshape(1),  # the device buffer Trainer.step returns
+           "theta_sample": theta[idx.to(theta.device)], "mixer_w": coord.w}
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -219,6 +252,7 @@ def run_ours(args) -> dict:
     phases = coord.timer.summary()
     rounds = coord.round - rounds0
     eager_launches = ops.launch_count() - c0
+    outputs = capture_outputs(trainer, coord) if args.dump_outputs and rank == 0 else None
     launches = K * trainer.launches_per_step + (eager_launches if trainer.use_graph else eager_launches - K * trainer.launches_per_step)
     tokens = K * B * T * world
     desc = GPT2_SMALL_DESC if trainer.cfg.name == "gpt2" else f"{trainer.cfg.name} ({trainer.man.num_params} params, vocab {V})"
@@ -310,6 +344,8 @@ def run_ours(args) -> dict:
     result["base_checksum"] = {"rank0": allc[0], "identical_on_all_ranks": bool(all(c == allc[0] for c in allc))}
     if hasattr(ex, "win"):
         ex.win.check_errors()
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if dist.is_initialized():
         dist.destroy_process_group()
     return result if rank == 0 else {}
@@ -317,6 +353,8 @@ def run_ours(args) -> dict:
 
 def main():
     args = parse_args()
+    if args.dump_outputs and args.impl in ("reference", "torch-bf16"):
+        raise SystemExit(f"--dump-outputs is not implemented for --impl {args.impl}")
     if args.impl == "reference":
         sys.path.insert(0, os.path.join(ROOT, "baseline"))
         from baseline.reference_arm import run_reference
