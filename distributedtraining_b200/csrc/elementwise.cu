@@ -728,8 +728,9 @@ __global__ void swiglu_bwd_kernel(const bf16* __restrict__ dout, const bf16* __r
   }
 }
 // rotate-half RoPE applied in place to the q and k heads of packed qkv [M, (H+2Hkv)*hd]; one thread per (row, head, pair).
+// inv_freq (optional, fp32 [hd/2]): precomputed inverse frequencies (scaled RoPE, e.g. Llama 3); nullptr = theta^(-2p/hd) inline.
 __global__ void rope_kernel(bf16* __restrict__ qkv, int M, int T, int nheads_rot, int row_stride, int hd, float log2_theta,
-                            float sign) {
+                            float sign, const float* __restrict__ inv_freq) {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   const int half = hd / 2;
   const size_t total = size_t(M) * nheads_rot * half;
@@ -738,7 +739,7 @@ __global__ void rope_kernel(bf16* __restrict__ qkv, int M, int T, int nheads_rot
     const int h = (i / half) % nheads_rot;
     const size_t row = i / (size_t(half) * nheads_rot);
     const int t = row % T;
-    const float inv = exp2f(-log2_theta * float(p) / float(half));
+    const float inv = inv_freq ? __ldg(inv_freq + p) : exp2f(-log2_theta * float(p) / float(half));
     float s, c;
     sincosf(float(t) * inv, &s, &c);
     s *= sign;
@@ -969,8 +970,9 @@ extern "C" int dtb_swiglu_bwd(const void* dout, const void* gu, void* dgu, int M
   return KCHECK();
 }
 extern "C" int dtb_rope(void* qkv, int M, int T, int nheads_rot, int row_stride, int hd, float theta, int inverse, int num_sms,
-                        cudaStream_t s) {
-  rope_kernel<<<num_sms * 8, 256, 0, s>>>((bf16*)qkv, M, T, nheads_rot, row_stride, hd, log2f(theta), inverse ? -1.f : 1.f);
+                        cudaStream_t s, const float* inv_freq) {
+  rope_kernel<<<num_sms * 8, 256, 0, s>>>((bf16*)qkv, M, T, nheads_rot, row_stride, hd, log2f(theta), inverse ? -1.f : 1.f,
+                                          inv_freq);
   return KCHECK();
 }
 extern "C" int dtb_quant_fp8(const void* x, void* q, const float* scale_in, float* amax_out, size_t n, int num_sms, cudaStream_t s,

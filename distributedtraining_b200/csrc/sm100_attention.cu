@@ -1,6 +1,9 @@
 // Causal self-attention for sm_100a on the 5th-gen tensor cores (tcgen05.mma, accumulators in TMEM, operands by TMA).
 //
-// Layout: packed qkv [M = B*T, (H + 2*Hkv) * 64] bf16 (q heads | k heads | v heads), head_dim = 64.
+// Layout: packed qkv [M = B*T, (H + 2*Hkv) * hd] bf16 (q heads | k heads | v heads), head_dim hd in {64, 128}: every kernel
+// is a template over HD.  An operand tile [128 rows x HD] is HD / 64 consecutive 128B-swizzle atoms [128 x 64] (16 KB each),
+// loaded as HD / 64 TMA boxes; K-major products over hd step (k >> 2) atoms + (k & 3) * 32 B, MN-major operands with N = HD
+// use LBO = atom stride (the same addressing as the two-atom P tile).
 // Tokens are treated as ONE flat axis of M rows cut into 128-row blocks; the mask is
 //        valid(r, c)  <=>  seq_start(r) <= c <= r            (same sequence AND causal)
 // so short sequences (the reference miner trains on T = 64: reference neurons/miner.py:70) are packed two per tile and
@@ -31,15 +34,15 @@ int make_tmap_2d(CUtensorMap* out, const void* ptr, int elem_bytes, uint64_t inn
                  uint32_t box_inner, uint32_t box_outer);  // sm100_gemm.cu
 
 constexpr int kBlk = 128;        // token rows per block (q and kv)
-constexpr int kHd = 64;          // head dim
-constexpr int kTile = kBlk * kHd * 2;  // 16 KB: one [128 x 64] bf16 tile (one 128B-swizzle atom wide)
+constexpr int kTile = kBlk * 64 * 2;  // 16 KB: one [128 x 64] bf16 128B-swizzle atom (a head-dim-64 tile, half of a 128 one)
+constexpr int kSmemLimit = 232448;     // 227 KB of dynamic shared memory per block
 constexpr float kLog2e = 1.4426950408889634f;
 
 struct AttnParams {
   CUtensorMap tmap_qkv;  // [M, qkv_dim], box 64 x 128
-  CUtensorMap tmap_do;   // [M, H*64],   box 64 x 128 (backward)
-  CUtensorMap tmap_o;    // [M, H*64],   box 64 x 128 (backward, single-block kernel: O tile for D = rowsum(dO * O))
-  CUtensorMap tmap_out;  // forward: out [M, H*64]; backward: dqkv [M, qkv_dim]; box 64 x 128 (single-block kernels store by TMA)
+  CUtensorMap tmap_do;   // [M, H*hd],   box 64 x 128 (backward)
+  CUtensorMap tmap_o;    // [M, H*hd],   box 64 x 128 (backward, single-block kernel: O tile for D = rowsum(dO * O))
+  CUtensorMap tmap_out;  // forward: out [M, H*hd]; backward: dqkv [M, qkv_dim]; box 64 x 128 (single-block kernels store by TMA)
   const __nv_bfloat16* o;
   const __nv_bfloat16* dout;
   __nv_bfloat16* out;    // forward output / backward dqkv
@@ -103,6 +106,19 @@ DTB_DEVICE void tmem_ld32x2(uint32_t ta, float* a, uint32_t tb, float* b) {
 DTB_DEVICE void st_swz(uint8_t* tile, int row, int ch, uint4 v) {
   *reinterpret_cast<uint4*>(tile + row * 128 + ((ch ^ (row & 7)) << 4)) = v;
 }
+// one [128 x HD] operand tile = HD / 64 TMA boxes (atoms) at columns col, col + 64, ...
+template <int HD>
+DTB_DEVICE void tma_load_tile(uint8_t* dst, const CUtensorMap* map, uint64_t* bar, int col, int row) {
+#pragma unroll
+  for (int a = 0; a < HD / 64; ++a) tma_load_2d(dst + a * kTile, map, bar, col + a * 64, row);
+}
+template <int HD>
+DTB_DEVICE void tma_store_tile(const CUtensorMap* map, uint8_t* src, int col, int row) {
+#pragma unroll
+  for (int a = 0; a < HD / 64; ++a) tma_store_2d(map, src + a * kTile, col + a * 64, row);
+}
+// descriptor offset (16 B units) of K-step k (16 bf16 = 32 B) of a K-major operand whose K extent spans 64-column atoms
+DTB_DEVICE constexpr uint64_t kstep_off(int k) { return uint64_t((k >> 2) * (kTile >> 4) + (k & 3) * 2); }
 
 // ---- softmax building blocks (one thread = one query row, 32-column chunks read from TMEM) -------------------------
 // ncu of the T = 512 kernels (profiles/ncu_r2_attn_tiled.md): 27 SASS instructions per score, 25 % issue utilisation at 2 warps
@@ -159,17 +175,22 @@ constexpr uint32_t kFullWarp = 0xffffffffu;
 // ------------------------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------------------------
-// smem: Q | K0 V0 | K1 V1 | P(2 atoms)   = 16 + 64 + 32 = 112 KB  -> 2 CTAs / SM;  TMEM: S[128] | O[64] -> 256 columns
-constexpr int kFwdSmem = 1024 + kTile * 7 + 64;
+// smem: Q | K0 V0 | K1 V1 | P(2 atoms)   hd 64: 16 + 64 + 32 = 112 KB -> 2 CTAs / SM;  hd 128: 32 + 128 + 32 = 192 KB -> 1
+// TMEM: S[128] | O[hd] -> 256 columns.  The output row is accumulated in registers (acc[HD]).
+template <int HD>
+constexpr int fwd_smem() { return 1024 + kTile * (5 * (HD / 64) + 2) + 64; }
+static_assert(fwd_smem<64>() <= kSmemLimit / 2 && fwd_smem<128>() <= kSmemLimit, "attn_fwd smem budget");
 
-__global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant__ AttnParams p) {
+template <int HD>
+__global__ void __launch_bounds__(128, HD == 64 ? 2 : 1) attn_fwd_kernel(const __grid_constant__ AttnParams p) {
+  constexpr int kOp = kTile * (HD / 64);  // one [128 x HD] operand tile
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;
-  uint8_t* sKV = smem + kTile;       // [2 stages][K, V]
-  uint8_t* sP = smem + kTile * 5;    // 2 atoms (keys 0-63 | 64-127)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kTile * 7);
+  uint8_t* sKV = smem + kOp;         // [2 stages][K, V]
+  uint8_t* sP = smem + kOp * 5;      // 2 atoms (keys 0-63 | 64-127)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOp * 5 + 2 * kTile);
   uint64_t* bar_q = bars;            // Q landed
   uint64_t* bar_kv = bars + 1;       // [2] K/V stage landed
   uint64_t* bar_s = bars + 3;        // S ready
@@ -185,7 +206,7 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
   const int seq_start = (row_tok / p.T) * p.T;
   const int kb_first = ((q0 / p.T) * p.T) / kBlk;  // kv block holding the start of the first row's sequence
   const int nkb = qb - kb_first + 1;
-  const int colQ = h * kHd, colK = (p.H + hk) * kHd, colV = (p.H + p.Hkv + hk) * kHd;
+  const int colQ = h * HD, colK = (p.H + hk) * HD, colV = (p.H + p.Hkv + hk) * HD;
 
   if (tid == 0) {
     tma_prefetch_desc(&p.tmap_qkv);
@@ -208,41 +229,41 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
   const uint32_t lane_off = (uint32_t(warp) * 32u) << 16;
 
   if (tid == 0) {
-    mbar_expect_tx(bar_q, kTile);
-    tma_load_2d(sQ, &p.tmap_qkv, bar_q, colQ, q0);
-    mbar_expect_tx(&bar_kv[0], 2 * kTile);
-    tma_load_2d(sKV, &p.tmap_qkv, &bar_kv[0], colK, kb_first * kBlk);
-    tma_load_2d(sKV + kTile, &p.tmap_qkv, &bar_kv[0], colV, kb_first * kBlk);
+    mbar_expect_tx(bar_q, kOp);
+    tma_load_tile<HD>(sQ, &p.tmap_qkv, bar_q, colQ, q0);
+    mbar_expect_tx(&bar_kv[0], 2 * kOp);
+    tma_load_tile<HD>(sKV, &p.tmap_qkv, &bar_kv[0], colK, kb_first * kBlk);
+    tma_load_tile<HD>(sKV + kOp, &p.tmap_qkv, &bar_kv[0], colV, kb_first * kBlk);
   }
 
   constexpr uint32_t idesc_s = make_idesc(kFmtBF16, kFmtBF16, false, false, 128, 128);
-  constexpr uint32_t idesc_o = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, 64);
+  constexpr uint32_t idesc_o = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, HD);
   const float sl2 = p.scale * kLog2e;
   const uint32_t dthr = p.drop.thr, rowkey = attn_row_key(p, h, row_tok);
   float m_run = -CUDART_INF_F, l_run = 0.f;
-  float acc[kHd];
+  float acc[HD];
 #pragma unroll
-  for (int i = 0; i < kHd; ++i) acc[i] = 0.f;
+  for (int i = 0; i < HD; ++i) acc[i] = 0.f;
 
   mbar_wait(bar_q, 0);
   for (int it = 0; it < nkb; ++it) {
     const int st = it & 1;
     const int k0 = (kb_first + it) * kBlk;
-    uint8_t* sK = sKV + st * 2 * kTile;
-    uint8_t* sV = sK + kTile;
+    uint8_t* sK = sKV + st * 2 * kOp;
+    uint8_t* sV = sK + kOp;
     if (tid == 0) {
       if (it + 1 < nkb) {  // prefetch the next K/V block into the other stage (its readers finished last iteration)
-        uint8_t* nK = sKV + (st ^ 1) * 2 * kTile;
-        mbar_expect_tx(&bar_kv[st ^ 1], 2 * kTile);
-        tma_load_2d(nK, &p.tmap_qkv, &bar_kv[st ^ 1], colK, k0 + kBlk);
-        tma_load_2d(nK + kTile, &p.tmap_qkv, &bar_kv[st ^ 1], colV, k0 + kBlk);
+        uint8_t* nK = sKV + (st ^ 1) * 2 * kOp;
+        mbar_expect_tx(&bar_kv[st ^ 1], 2 * kOp);
+        tma_load_tile<HD>(nK, &p.tmap_qkv, &bar_kv[st ^ 1], colK, k0 + kBlk);
+        tma_load_tile<HD>(nK + kOp, &p.tmap_qkv, &bar_kv[st ^ 1], colV, k0 + kBlk);
       }
       mbar_wait(&bar_kv[st], (it >> 1) & 1);
       tc_fence_after();
       const uint64_t dq = make_smem_desc(smem_u32(sQ), 16, 1024);
       const uint64_t dk = make_smem_desc(smem_u32(sK), 16, 1024);
 #pragma unroll
-      for (int k = 0; k < kHd / 16; ++k) umma_f16(tS, dq + uint64_t(k * 2), dk + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tS, dq + kstep_off(k), dk + kstep_off(k), idesc_s, k > 0);
       umma_commit(bar_s);
     }
     mbar_wait(bar_s, it & 1);
@@ -286,7 +307,7 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
     l_run = l_run * alpha + lsum;
     m_run = m_new;
 #pragma unroll
-    for (int i = 0; i < kHd; ++i) acc[i] *= alpha;
+    for (int i = 0; i < HD; ++i) acc[i] *= alpha;
     fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
@@ -303,7 +324,7 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
     mbar_wait(bar_o, it & 1);
     tc_fence_after();
 #pragma unroll
-    for (int ch = 0; ch < 2; ++ch) {
+    for (int ch = 0; ch < HD / 32; ++ch) {
       float o[32];
       tmem_ld32(tO + lane_off + ch * 32, o);
 #pragma unroll
@@ -316,11 +337,11 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
   {
     const float inv = l_run > 0.f ? 1.f / l_run : 0.f;  // rows >= M: all masked -> zeros, clipped by the tensor map anyway
 #pragma unroll
-    for (int v = 0; v < 8; ++v) {
+    for (int v = 0; v < HD / 8; ++v) {
       uint4 q;
       q.x = pack2(acc[v * 8 + 0] * inv, acc[v * 8 + 1] * inv); q.y = pack2(acc[v * 8 + 2] * inv, acc[v * 8 + 3] * inv);
       q.z = pack2(acc[v * 8 + 4] * inv, acc[v * 8 + 5] * inv); q.w = pack2(acc[v * 8 + 6] * inv, acc[v * 8 + 7] * inv);
-      st_swz(sQ, tid, v, q);
+      st_swz(sQ + (v >> 3) * kTile, tid, v & 7, q);
     }
     fence_proxy_async_smem();
     if (row_tok < p.M && p.lse) {
@@ -332,7 +353,7 @@ __global__ void __launch_bounds__(128, 2) attn_fwd_kernel(const __grid_constant_
   __syncthreads();
   if (warp == 0) {
     if (elect_one()) {
-      tma_store_2d(&p.tmap_out, sQ, h * kHd, q0);
+      tma_store_tile<HD>(&p.tmap_out, sQ, h * HD, q0);
       tma_store_commit();
       tma_store_wait_read<0>();
     }
@@ -411,14 +432,15 @@ DTB_DEVICE void bwd_softmax_tiles(uint32_t tS, uint32_t tDP, uint32_t lane_off, 
 }
 
 // D = rowsum(dO * O), lse in log2 units, for this thread's q row
+template <int HD>
 DTB_DEVICE void load_row_stats(const AttnParams& p, int row_tok, int h, float& Drow, float& lse_l2) {
   Drow = 0.f;
   lse_l2 = 0.f;
   if (row_tok < p.M) {
-    const uint4* a = reinterpret_cast<const uint4*>(p.dout + size_t(row_tok) * p.ld_o + h * kHd);
-    const uint4* b = reinterpret_cast<const uint4*>(p.o + size_t(row_tok) * p.ld_o + h * kHd);
+    const uint4* a = reinterpret_cast<const uint4*>(p.dout + size_t(row_tok) * p.ld_o + h * HD);
+    const uint4* b = reinterpret_cast<const uint4*>(p.o + size_t(row_tok) * p.ld_o + h * HD);
 #pragma unroll
-    for (int v = 0; v < 8; ++v) {
+    for (int v = 0; v < HD / 8; ++v) {
       const uint4 x = __ldg(a + v), y = __ldg(b + v);
       const __nv_bfloat162* xh = reinterpret_cast<const __nv_bfloat162*>(&x);
       const __nv_bfloat162* yh = reinterpret_cast<const __nv_bfloat162*>(&y);
@@ -433,15 +455,16 @@ DTB_DEVICE void load_row_stats(const AttnParams& p, int row_tok, int h, float& D
   }
 }
 
-// Same statistics from the TMA-loaded dO / O tiles in shared memory (128B-swizzled [128 x 64] bf16): replaces 16 row-strided
+// Same statistics from the TMA-loaded dO / O tiles in shared memory (128B-swizzled [128 x HD] bf16): replaces 16 row-strided
 // LDG.128 per thread (17 % of the single-block kernel's stall samples sat on their first use) with conflict-free LDS.
+template <int HD>
 DTB_DEVICE void row_stats_smem(const AttnParams& p, const uint8_t* sDO, const uint8_t* sO, int row, int row_tok, int h, float& Drow,
                                float& lse_l2) {
   Drow = 0.f;
   lse_l2 = 0.f;
 #pragma unroll
-  for (int ch = 0; ch < 8; ++ch) {
-    const uint32_t off = row * 128 + ((ch ^ (row & 7)) << 4);
+  for (int ch = 0; ch < HD / 8; ++ch) {
+    const uint32_t off = (ch >> 3) * kTile + row * 128 + (((ch & 7) ^ (row & 7)) << 4);
     const uint4 x = *reinterpret_cast<const uint4*>(sDO + off), y = *reinterpret_cast<const uint4*>(sO + off);
     const __nv_bfloat162* xh = reinterpret_cast<const __nv_bfloat162*>(&x);
     const __nv_bfloat162* yh = reinterpret_cast<const __nv_bfloat162*>(&y);
@@ -457,21 +480,30 @@ DTB_DEVICE void row_stats_smem(const AttnParams& p, const uint8_t* sDO, const ui
   }
 }
 
-// --- KV-owner kernel: grid (kv-block, kv-head).  smem: K V | (Q dO) x2 | P(2) | dS(2) = 32+64+32+32 = 160 KB ---
-constexpr int kBwdKvSmem = 1024 + kTile * 10 + 128;
+// --- KV-owner kernel: grid (kv-block, kv-head).  smem: K V | (Q dO) x stages | P(2) | dS(2)
+//     hd 64: 32 + 2 x 32 + 32 + 32 = 160 KB;  hd 128: 64 + 1 x 64 + 32 + 32 = 192 KB (two Q/dO stages would need 256 KB)
+// TMEM: S[128] dP[128] dV[hd] dK[hd] -> 512 columns at hd 128 (all of them)
+template <int HD>
+constexpr int bwd_kv_stages() { return HD == 64 ? 2 : 1; }
+template <int HD>
+constexpr int bwd_kv_smem() { return 1024 + kTile * (2 * (HD / 64) + bwd_kv_stages<HD>() * 2 * (HD / 64) + 4) + 128; }
+static_assert(bwd_kv_smem<64>() <= kSmemLimit && bwd_kv_smem<128>() <= kSmemLimit, "attn_bwd_kv smem budget");
+static_assert(256 + 2 * 128 <= 512, "attn_bwd_kv TMEM budget");
 
+template <int HD>
 __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_constant__ AttnParams p) {
+  constexpr int kOp = kTile * (HD / 64), kSt = bwd_kv_stages<HD>();
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sK = smem;
-  uint8_t* sV = smem + kTile;
-  uint8_t* sQD = smem + 2 * kTile;  // [2 stages][Q, dO]
-  uint8_t* sP = smem + 6 * kTile;
-  uint8_t* sDS = smem + 8 * kTile;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 10 * kTile);
+  uint8_t* sV = smem + kOp;
+  uint8_t* sQD = smem + 2 * kOp;  // [kSt stages][Q, dO]
+  uint8_t* sP = sQD + kSt * 2 * kOp;
+  uint8_t* sDS = sP + 2 * kTile;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sDS + 2 * kTile);
   uint64_t* bar_kv = bars;
-  uint64_t* bar_qd = bars + 1;  // [2]
+  uint64_t* bar_qd = bars + 1;  // [2] (one used with a single stage)
   uint64_t* bar_s = bars + 3;
   uint64_t* bar_g = bars + 4;   // dV/dK MMAs of this iteration done (P/dS/Q/dO buffers reusable)
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 5);
@@ -487,7 +519,7 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_consta
   const int qb_last = (min(seq_end, p.M) - 1) / kBlk;
   const int nqb = qb_last - kb + 1;
   const int niter = nqb * group;
-  const int colK = (p.H + hk) * kHd, colV = (p.H + p.Hkv + hk) * kHd;
+  const int colK = (p.H + hk) * HD, colV = (p.H + p.Hkv + hk) * HD;
 
   if (tid == 0) {
     tma_prefetch_desc(&p.tmap_qkv);
@@ -507,50 +539,50 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_consta
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr;
-  const uint32_t tS = tmem, tDP = tmem + 128, tDV = tmem + 256, tDK = tmem + 320;
+  const uint32_t tS = tmem, tDP = tmem + 128, tDV = tmem + 256, tDK = tmem + 256 + HD;
   const uint32_t lane_off = (uint32_t(warp) * 32u) << 16;
 
   auto issue_qd = [&](int it) {
-    const int st = it & 1;
+    const int st = kSt == 2 ? (it & 1) : 0;
     const int hq = hk * group + it % group;
     const int q0 = (kb + it / group) * kBlk;
-    uint8_t* dst = sQD + st * 2 * kTile;
-    mbar_expect_tx(&bar_qd[st], 2 * kTile);
-    tma_load_2d(dst, &p.tmap_qkv, &bar_qd[st], hq * kHd, q0);
-    tma_load_2d(dst + kTile, &p.tmap_do, &bar_qd[st], hq * kHd, q0);
+    uint8_t* dst = sQD + st * 2 * kOp;
+    mbar_expect_tx(&bar_qd[st], 2 * kOp);
+    tma_load_tile<HD>(dst, &p.tmap_qkv, &bar_qd[st], hq * HD, q0);
+    tma_load_tile<HD>(dst + kOp, &p.tmap_do, &bar_qd[st], hq * HD, q0);
   };
   if (tid == 0) {
-    mbar_expect_tx(bar_kv, 2 * kTile);
-    tma_load_2d(sK, &p.tmap_qkv, bar_kv, colK, k0);
-    tma_load_2d(sV, &p.tmap_qkv, bar_kv, colV, k0);
+    mbar_expect_tx(bar_kv, 2 * kOp);
+    tma_load_tile<HD>(sK, &p.tmap_qkv, bar_kv, colK, k0);
+    tma_load_tile<HD>(sV, &p.tmap_qkv, bar_kv, colV, k0);
     issue_qd(0);
   }
   constexpr uint32_t idesc_s = make_idesc(kFmtBF16, kFmtBF16, false, false, 128, 128);   // S, dP
-  constexpr uint32_t idesc_g = make_idesc(kFmtBF16, kFmtBF16, true, true, 128, 64);      // dV = P^T dO, dK = dS^T Q
+  constexpr uint32_t idesc_g = make_idesc(kFmtBF16, kFmtBF16, true, true, 128, HD);      // dV = P^T dO, dK = dS^T Q
   const float sl2 = p.scale * kLog2e;
   mbar_wait(bar_kv, 0);
 
   for (int it = 0; it < niter; ++it) {
-    const int st = it & 1;
+    const int st = kSt == 2 ? (it & 1) : 0;
     const int hq = hk * group + it % group;
     const int q0 = (kb + it / group) * kBlk;
-    uint8_t* sQ = sQD + st * 2 * kTile;
-    uint8_t* sDO = sQ + kTile;
+    uint8_t* sQ = sQD + st * 2 * kOp;
+    uint8_t* sDO = sQ + kOp;
     if (tid == 0) {
-      if (it + 1 < niter) issue_qd(it + 1);  // other stage: its MMAs completed (bar_g of iteration it-1)
-      mbar_wait(&bar_qd[st], (it >> 1) & 1);
+      if (kSt == 2 && it + 1 < niter) issue_qd(it + 1);  // other stage: its MMAs completed (bar_g of iteration it-1)
+      mbar_wait(&bar_qd[st], kSt == 2 ? ((it >> 1) & 1) : (it & 1));
       tc_fence_after();
       const uint64_t dq = make_smem_desc(smem_u32(sQ), 16, 1024), dk = make_smem_desc(smem_u32(sK), 16, 1024);
       const uint64_t ddo = make_smem_desc(smem_u32(sDO), 16, 1024), dv = make_smem_desc(smem_u32(sV), 16, 1024);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tS, dq + uint64_t(k * 2), dk + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tS, dq + kstep_off(k), dk + kstep_off(k), idesc_s, k > 0);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tDP, ddo + uint64_t(k * 2), dv + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tDP, ddo + kstep_off(k), dv + kstep_off(k), idesc_s, k > 0);
       umma_commit(bar_s);
     }
     const int row_tok = q0 + tid;
     float Drow, lse_l2;
-    load_row_stats(p, row_tok, hq, Drow, lse_l2);
+    load_row_stats<HD>(p, row_tok, hq, Drow, lse_l2);
     const int seq_start = (row_tok / p.T) * p.T;
     const int c_lo = seq_start - k0, c_hi = row_last_key(p, row_tok) - k0;
     mbar_wait(bar_s, it & 1);
@@ -580,6 +612,7 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_consta
     }
     mbar_wait(bar_g, it & 1);  // smem tiles + S/dP TMEM free for the next iteration
     tc_fence_after();
+    if (kSt == 1 && tid == 0 && it + 1 < niter) issue_qd(it + 1);  // single stage: refill once this iteration's MMAs are done
   }
   // ---- write dK, dV (thread = key row).  tcgen05.ld is warp-collective: loads are unconditional, stores guarded ----
   const int key_tok = k0 + tid;
@@ -588,7 +621,7 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_consta
     const uint32_t t = which == 0 ? tDK : tDV;
     __nv_bfloat16* dst = p.out + size_t(key_tok) * p.ld_out + (which == 0 ? colK : colV);
 #pragma unroll
-    for (int ch = 0; ch < 2; ++ch) {
+    for (int ch = 0; ch < HD / 32; ++ch) {
       float o[32];
       tmem_ld32(t + lane_off + ch * 32, o);
       if (key_tok < p.M) {
@@ -610,18 +643,23 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_kv_kernel(const __grid_consta
   }
 }
 
-// --- Q-owner kernel: grid (q-block, head).  smem: Q dO | (K V) x2 | dS(2) = 32+64+32 = 128 KB ---
-constexpr int kBwdQSmem = 1024 + kTile * 8 + 128;
+// --- Q-owner kernel: grid (q-block, head).  smem: Q dO | (K V) x2 | dS(2) = 32+64+32 = 128 KB (hd 128: 64+128+32 = 224 KB) ---
+// TMEM: S[128] dP[128] dQ[hd] -> 512 columns allocated
+template <int HD>
+constexpr int bwd_q_smem() { return 1024 + kTile * (6 * (HD / 64) + 2) + 128; }
+static_assert(bwd_q_smem<64>() <= kSmemLimit && bwd_q_smem<128>() <= kSmemLimit, "attn_bwd_q smem budget");
 
+template <int HD>
 __global__ void __launch_bounds__(128, 1) attn_bwd_q_kernel(const __grid_constant__ AttnParams p) {
+  constexpr int kOp = kTile * (HD / 64);
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;
-  uint8_t* sDO = smem + kTile;
-  uint8_t* sKV = smem + 2 * kTile;
-  uint8_t* sDS = smem + 6 * kTile;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 8 * kTile);
+  uint8_t* sDO = smem + kOp;
+  uint8_t* sKV = smem + 2 * kOp;
+  uint8_t* sDS = smem + 6 * kOp;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sDS + 2 * kTile);
   uint64_t* bar_q = bars;
   uint64_t* bar_kv = bars + 1;  // [2]
   uint64_t* bar_s = bars + 3;
@@ -637,7 +675,7 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_q_kernel(const __grid_constan
   const int seq_start = (row_tok / p.T) * p.T;
   const int kb_first = ((q0 / p.T) * p.T) / kBlk;
   const int nkb = qb - kb_first + 1;
-  const int colK = (p.H + hk) * kHd, colV = (p.H + p.Hkv + hk) * kHd;
+  const int colK = (p.H + hk) * HD, colV = (p.H + p.Hkv + hk) * HD;
 
   if (tid == 0) {
     tma_prefetch_desc(&p.tmap_qkv);
@@ -661,41 +699,41 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_q_kernel(const __grid_constan
   const uint32_t lane_off = (uint32_t(warp) * 32u) << 16;
 
   if (tid == 0) {
-    mbar_expect_tx(bar_q, 2 * kTile);
-    tma_load_2d(sQ, &p.tmap_qkv, bar_q, h * kHd, q0);
-    tma_load_2d(sDO, &p.tmap_do, bar_q, h * kHd, q0);
-    mbar_expect_tx(&bar_kv[0], 2 * kTile);
-    tma_load_2d(sKV, &p.tmap_qkv, &bar_kv[0], colK, kb_first * kBlk);
-    tma_load_2d(sKV + kTile, &p.tmap_qkv, &bar_kv[0], colV, kb_first * kBlk);
+    mbar_expect_tx(bar_q, 2 * kOp);
+    tma_load_tile<HD>(sQ, &p.tmap_qkv, bar_q, h * HD, q0);
+    tma_load_tile<HD>(sDO, &p.tmap_do, bar_q, h * HD, q0);
+    mbar_expect_tx(&bar_kv[0], 2 * kOp);
+    tma_load_tile<HD>(sKV, &p.tmap_qkv, &bar_kv[0], colK, kb_first * kBlk);
+    tma_load_tile<HD>(sKV + kOp, &p.tmap_qkv, &bar_kv[0], colV, kb_first * kBlk);
   }
   constexpr uint32_t idesc_s = make_idesc(kFmtBF16, kFmtBF16, false, false, 128, 128);
-  constexpr uint32_t idesc_q = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, 64);  // dQ = dS K  (B = K, MN-major)
+  constexpr uint32_t idesc_q = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, HD);  // dQ = dS K  (B = K, MN-major)
   const float sl2 = p.scale * kLog2e;
   const uint32_t rowkey = attn_row_key(p, h, row_tok);
   float Drow, lse_l2;
-  load_row_stats(p, row_tok, h, Drow, lse_l2);
+  load_row_stats<HD>(p, row_tok, h, Drow, lse_l2);
   mbar_wait(bar_q, 0);
 
   for (int it = 0; it < nkb; ++it) {
     const int st = it & 1;
     const int k0 = (kb_first + it) * kBlk;
-    uint8_t* sK = sKV + st * 2 * kTile;
-    uint8_t* sV = sK + kTile;
+    uint8_t* sK = sKV + st * 2 * kOp;
+    uint8_t* sV = sK + kOp;
     if (tid == 0) {
       if (it + 1 < nkb) {
-        uint8_t* nK = sKV + (st ^ 1) * 2 * kTile;
-        mbar_expect_tx(&bar_kv[st ^ 1], 2 * kTile);
-        tma_load_2d(nK, &p.tmap_qkv, &bar_kv[st ^ 1], colK, k0 + kBlk);
-        tma_load_2d(nK + kTile, &p.tmap_qkv, &bar_kv[st ^ 1], colV, k0 + kBlk);
+        uint8_t* nK = sKV + (st ^ 1) * 2 * kOp;
+        mbar_expect_tx(&bar_kv[st ^ 1], 2 * kOp);
+        tma_load_tile<HD>(nK, &p.tmap_qkv, &bar_kv[st ^ 1], colK, k0 + kBlk);
+        tma_load_tile<HD>(nK + kOp, &p.tmap_qkv, &bar_kv[st ^ 1], colV, k0 + kBlk);
       }
       mbar_wait(&bar_kv[st], (it >> 1) & 1);
       tc_fence_after();
       const uint64_t dq = make_smem_desc(smem_u32(sQ), 16, 1024), dk = make_smem_desc(smem_u32(sK), 16, 1024);
       const uint64_t ddo = make_smem_desc(smem_u32(sDO), 16, 1024), dv = make_smem_desc(smem_u32(sV), 16, 1024);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tS, dq + uint64_t(k * 2), dk + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tS, dq + kstep_off(k), dk + kstep_off(k), idesc_s, k > 0);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tDP, ddo + uint64_t(k * 2), dv + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tDP, ddo + kstep_off(k), dv + kstep_off(k), idesc_s, k > 0);
       umma_commit(bar_s);
     }
     const int c_lo = seq_start - k0, c_hi = row_last_key(p, row_tok) - k0;
@@ -719,12 +757,13 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_q_kernel(const __grid_constan
     mbar_wait(bar_g, it & 1);
     tc_fence_after();
   }
-  {
+#pragma unroll
+  for (int c2 = 0; c2 < HD / 64; ++c2) {
     float o0[32], o1[32];
-    tmem_ld32(tDQ + lane_off, o0);
-    tmem_ld32(tDQ + lane_off + 32, o1);
+    tmem_ld32(tDQ + lane_off + c2 * 64, o0);
+    tmem_ld32(tDQ + lane_off + c2 * 64 + 32, o1);
     if (row_tok < p.M) {
-      __nv_bfloat16* dst = p.out + size_t(row_tok) * p.ld_out + h * kHd;
+      __nv_bfloat16* dst = p.out + size_t(row_tok) * p.ld_out + h * HD + c2 * 64;
 #pragma unroll
       for (int v = 0; v < 4; ++v) {
         uint4 q;
@@ -748,19 +787,23 @@ __global__ void __launch_bounds__(128, 1) attn_bwd_q_kernel(const __grid_constan
 // ------------------------------------------------------------------------------------------------------------------
 // single-block fast paths: every 128-token block is self-contained (128 % T == 0 or T == 128: the reference miner's T = 64)
 // ------------------------------------------------------------------------------------------------------------------
-// forward: Q K V | P aliases Q+K (dead once S is computed);  TMEM: S[128], O reuses S[0:64]  -> 48 KB + 128 columns,
-// four CTAs per SM overlap each other's TMA / MMA / softmax phases.
-constexpr int kFwdSmallSmem = 1024 + kTile * 3 + 64;
+// forward: Q K V | P aliases the first two atoms (Q+K at hd 64, Q at hd 128: dead once S is computed);  TMEM: S[128], O reuses
+// S[0:hd]  -> hd 64: 48 KB + 128 columns, four CTAs per SM overlap each other's TMA / MMA / softmax phases; hd 128: 96 KB, two.
+template <int HD>
+constexpr int fwd_small_smem() { return 1024 + kTile * 3 * (HD / 64) + 64; }
+static_assert(fwd_small_smem<64>() <= kSmemLimit / 4 && fwd_small_smem<128>() <= kSmemLimit / 2, "attn_fwd_small smem budget");
 
-__global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_constant__ AttnParams p) {
+template <int HD>
+__global__ void __launch_bounds__(128, HD == 64 ? 4 : 2) attn_fwd_small_kernel(const __grid_constant__ AttnParams p) {
+  constexpr int kOp = kTile * (HD / 64);
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;
-  uint8_t* sK = smem + kTile;
-  uint8_t* sV = smem + 2 * kTile;
-  uint8_t* sP = smem;  // 2 atoms over Q|K
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kTile * 3);
+  uint8_t* sK = smem + kOp;
+  uint8_t* sV = smem + 2 * kOp;
+  uint8_t* sP = smem;  // 2 atoms over Q|K (hd 64) or Q (hd 128)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOp * 3);
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 3);
   const int tid = threadIdx.x, warp = tid >> 5;
   const int qb = blockIdx.x, h = blockIdx.y;
@@ -785,20 +828,20 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
   const uint32_t tmem = *tmem_ptr;
   const uint32_t lane_off = (uint32_t(warp) * 32u) << 16;
   constexpr uint32_t idesc_s = make_idesc(kFmtBF16, kFmtBF16, false, false, 128, 128);
-  constexpr uint32_t idesc_o = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, 64);
+  constexpr uint32_t idesc_o = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, HD);
   if (warp == 0) {  // warp-uniform issue: only the instructions themselves sit under elect.sync (see sm100_gemm.cu)
     if (elect_one()) {
-      mbar_expect_tx(&bars[0], 3 * kTile);
-      tma_load_2d(sQ, &p.tmap_qkv, &bars[0], h * kHd, q0);
-      tma_load_2d(sK, &p.tmap_qkv, &bars[0], (p.H + hk) * kHd, q0);
-      tma_load_2d(sV, &p.tmap_qkv, &bars[0], (p.H + p.Hkv + hk) * kHd, q0);
+      mbar_expect_tx(&bars[0], 3 * kOp);
+      tma_load_tile<HD>(sQ, &p.tmap_qkv, &bars[0], h * HD, q0);
+      tma_load_tile<HD>(sK, &p.tmap_qkv, &bars[0], (p.H + hk) * HD, q0);
+      tma_load_tile<HD>(sV, &p.tmap_qkv, &bars[0], (p.H + p.Hkv + hk) * HD, q0);
     }
     mbar_wait(&bars[0], 0);
     tc_fence_after();
     const uint64_t dq = make_smem_desc(smem_u32(sQ), 16, 1024), dk = make_smem_desc(smem_u32(sK), 16, 1024);
     if (elect_one()) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tmem, dq + uint64_t(k * 2), dk + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tmem, dq + kstep_off(k), dk + kstep_off(k), idesc_s, k > 0);
       umma_commit(&bars[1]);
     }
   }
@@ -857,7 +900,7 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
       for (int k = 0; k < kBlk / 16; ++k) {
         const uint64_t dp = make_smem_desc(pbase + (k >> 2) * kTile + (k & 3) * 32, 16, 1024);
         const uint64_t dv = make_smem_desc(vbase + k * 2048, kTile, 1024);
-        umma_f16(tmem, dp, dv, idesc_o, k > 0);  // O overwrites S[0:64] (every thread has consumed S)
+        umma_f16(tmem, dp, dv, idesc_o, k > 0);  // O overwrites S[0:hd] (every thread has consumed S)
       }
       umma_commit(&bars[2]);
     }
@@ -868,7 +911,7 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
   // O tile -> swizzled staging tile in the (dead) Q region -> ONE TMA store (rows >= M are clipped by the tensor map).
   // Per-thread 16 B global stores of 32 different rows per instruction throttled the LSU (lg_throttle, ncu).
 #pragma unroll
-  for (int ch = 0; ch < 2; ++ch) {
+  for (int ch = 0; ch < HD / 32; ++ch) {
     float o[32];
     tmem_ld32(tmem + lane_off + ch * 32, o);
 #pragma unroll
@@ -876,7 +919,7 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
       uint4 q;
       q.x = pack2(o[v * 8 + 0] * inv, o[v * 8 + 1] * inv); q.y = pack2(o[v * 8 + 2] * inv, o[v * 8 + 3] * inv);
       q.z = pack2(o[v * 8 + 4] * inv, o[v * 8 + 5] * inv); q.w = pack2(o[v * 8 + 6] * inv, o[v * 8 + 7] * inv);
-      st_swz(sQ, tid, ch * 4 + v, q);
+      st_swz(sQ + (ch >> 1) * kTile, tid, (ch & 1) * 4 + v, q);
     }
   }
   fence_proxy_async_smem();
@@ -888,7 +931,7 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
   __syncthreads();
   if (warp == 0) {
     if (elect_one()) {
-      tma_store_2d(&p.tmap_out, sQ, h * kHd, q0);
+      tma_store_tile<HD>(&p.tmap_out, sQ, h * HD, q0);
       tma_store_commit();
       tma_store_wait_read<0>();  // the staging tile must outlive the bulk read
     }
@@ -903,25 +946,31 @@ __global__ void __launch_bounds__(128, 4) attn_fwd_small_kernel(const __grid_con
 // smem: Q K dO | V -> P0 | P1 | dS(2) = 112 KB (P overwrites V, which is dead once dP is computed);
 // TMEM: S[128] dP[128], then dV/dK/dQ overwrite them (every thread has consumed S/dP) = 256 columns -> TWO CTAs per SM
 // overlap each other's TMA / MMA / softmax phases (the first version ran one CTA per SM at 6 % occupancy, 126 us/layer).
-constexpr int kBwdSmallSmem = kTile * 7 + 64;
+// hd 128: Q K dO | V = P(2) | dS(2) = 160 KB; dV/dK/dQ take 384 columns -> 512 allocated, one CTA per SM.
+template <int HD>
+constexpr int bwd_small_smem() { return kTile * (3 * (HD / 64) + 4) + 64; }
+static_assert(bwd_small_smem<64>() <= kSmemLimit / 2 && bwd_small_smem<128>() <= kSmemLimit, "attn_bwd_small smem budget");
 
-__global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_constant__ AttnParams p) {
+template <int HD>
+__global__ void __launch_bounds__(128, HD == 64 ? 2 : 1) attn_bwd_small_kernel(const __grid_constant__ AttnParams p) {
+  constexpr int kOp = kTile * (HD / 64);
+  constexpr uint32_t kCols = HD == 64 ? 256 : 512;  // TMEM columns
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent GEMM may start its prologue (sm100_ptx.cuh)
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw;  // the dynamic window starts 1 KB-aligned (no static shared memory in this kernel)
   uint8_t* sQ = smem;
-  uint8_t* sK = smem + kTile;
-  uint8_t* sDO = smem + 2 * kTile;
-  uint8_t* sV = smem + 3 * kTile;
-  uint8_t* sP = smem + 3 * kTile;   // aliases V
-  uint8_t* sDS = smem + 5 * kTile;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 7 * kTile);
+  uint8_t* sK = smem + kOp;
+  uint8_t* sDO = smem + 2 * kOp;
+  uint8_t* sV = smem + 3 * kOp;
+  uint8_t* sP = smem + 3 * kOp;     // aliases V
+  uint8_t* sDS = sP + 2 * kTile;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sDS + 2 * kTile);
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 3);
   const int tid = threadIdx.x, warp = tid >> 5;
   const int qb = blockIdx.x, h = blockIdx.y;
   const int q0 = qb * kBlk;
   const int row_tok = q0 + tid;
-  const int colQ = h * kHd, colK = (p.H + h) * kHd, colV = (2 * p.H + h) * kHd;
+  const int colQ = h * HD, colK = (p.H + h) * HD, colV = (2 * p.H + h) * HD;
   if (tid == 0) {
     tma_prefetch_desc(&p.tmap_qkv);
     tma_prefetch_desc(&p.tmap_do);
@@ -931,7 +980,7 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
     fence_barrier_init();
   }
   if (warp == 0) {
-    tmem_alloc(tmem_ptr, 256);
+    tmem_alloc(tmem_ptr, kCols);
     tmem_relinquish();
   }
   tc_fence_before();
@@ -940,20 +989,20 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
   pdl_wait();  // PDL: launched early -- everything above touched only shared memory / TMEM / kernel parameters
   const uint32_t tmem = *tmem_ptr;
   const uint32_t tS = tmem, tDP = tmem + 128;
-  const uint32_t tDV = tmem, tDK = tmem + 64, tDQ = tmem + 128;  // reuse S / dP after the softmax tiles are in smem
+  const uint32_t tDV = tmem, tDK = tmem + HD, tDQ = tmem + 2 * HD;  // reuse S / dP after the softmax tiles are in smem
   if ((smem_u32(smem_raw) & 1023u) != 0) __trap();  // layout assumption of the swizzled tiles
   const uint32_t lane_off = (uint32_t(warp) * 32u) << 16;
   constexpr uint32_t idesc_s = make_idesc(kFmtBF16, kFmtBF16, false, false, 128, 128);
-  constexpr uint32_t idesc_g = make_idesc(kFmtBF16, kFmtBF16, true, true, 128, 64);
-  constexpr uint32_t idesc_q = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, 64);
+  constexpr uint32_t idesc_g = make_idesc(kFmtBF16, kFmtBF16, true, true, 128, HD);
+  constexpr uint32_t idesc_q = make_idesc(kFmtBF16, kFmtBF16, false, true, 128, HD);
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(&bars[0], 5 * kTile);
-      tma_load_2d(sQ, &p.tmap_qkv, &bars[0], colQ, q0);
-      tma_load_2d(sK, &p.tmap_qkv, &bars[0], colK, q0);
-      tma_load_2d(sV, &p.tmap_qkv, &bars[0], colV, q0);
-      tma_load_2d(sDO, &p.tmap_do, &bars[0], colQ, q0);
-      tma_load_2d(sDS, &p.tmap_o, &bars[0], colQ, q0);  // O tile parks in the (still dead) dS region until D is formed
+      mbar_expect_tx(&bars[0], 5 * kOp);
+      tma_load_tile<HD>(sQ, &p.tmap_qkv, &bars[0], colQ, q0);
+      tma_load_tile<HD>(sK, &p.tmap_qkv, &bars[0], colK, q0);
+      tma_load_tile<HD>(sV, &p.tmap_qkv, &bars[0], colV, q0);
+      tma_load_tile<HD>(sDO, &p.tmap_do, &bars[0], colQ, q0);
+      tma_load_tile<HD>(sDS, &p.tmap_o, &bars[0], colQ, q0);  // O tile parks in the (still dead) dS region until D is formed
     }
     mbar_wait(&bars[0], 0);
     tc_fence_after();
@@ -961,16 +1010,16 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
     const uint64_t ddo = make_smem_desc(smem_u32(sDO), 16, 1024), dv = make_smem_desc(smem_u32(sV), 16, 1024);
     if (elect_one()) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tS, dq + uint64_t(k * 2), dk + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tS, dq + kstep_off(k), dk + kstep_off(k), idesc_s, k > 0);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tDP, ddo + uint64_t(k * 2), dv + uint64_t(k * 2), idesc_s, k > 0);
+      for (int k = 0; k < HD / 16; ++k) umma_f16(tDP, ddo + kstep_off(k), dv + kstep_off(k), idesc_s, k > 0);
       umma_commit(&bars[1]);
     }
   }
   float Drow, lse_l2;
   if (warp != 0) mbar_wait(&bars[0], 0);  // (warp 0 passed it before issuing the MMAs) the dO / O tiles have landed
   // each thread reads ITS row of the O tile here and overwrites only that same row of dS later: no barrier needed in between
-  row_stats_smem(p, sDO, sDS, tid, row_tok, h, Drow, lse_l2);
+  row_stats_smem<HD>(p, sDO, sDS, tid, row_tok, h, Drow, lse_l2);
   const int c_lo = (row_tok / p.T) * p.T - q0, c_hi = row_last_key(p, row_tok) - q0;
   mbar_wait(&bars[1], 0);
   tc_fence_after();
@@ -1008,9 +1057,9 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
 #pragma unroll 1
   for (int which = 0; which < 3; ++which) {
     const uint32_t t = which == 0 ? tDQ : (which == 1 ? tDK : tDV);
-    uint8_t* stage = smem + which * kTile;
+    uint8_t* stage = smem + which * kOp;
 #pragma unroll
-    for (int ch = 0; ch < 2; ++ch) {
+    for (int ch = 0; ch < HD / 32; ++ch) {
       float o[32];
       tmem_ld32(t + lane_off + ch * 32, o);
 #pragma unroll
@@ -1018,7 +1067,7 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
         uint4 q;
         q.x = pack2(o[v * 8 + 0], o[v * 8 + 1]); q.y = pack2(o[v * 8 + 2], o[v * 8 + 3]);
         q.z = pack2(o[v * 8 + 4], o[v * 8 + 5]); q.w = pack2(o[v * 8 + 6], o[v * 8 + 7]);
-        st_swz(stage, tid, ch * 4 + v, q);
+        st_swz(stage + (ch >> 1) * kTile, tid, (ch & 1) * 4 + v, q);
       }
     }
   }
@@ -1026,9 +1075,10 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
   tc_fence_before();
   __syncthreads();
   if (p.dbias) {
-    // qkv bias gradient folded in: column sums of the three staged [128 x 64] tiles (the bf16 values that are stored), one
-    // atomicAdd per column per CTA -- replaces a separate pass over dqkv (18 us per layer).  Thread t: tile t / 64 (and the
-    // third tile split by halves), column t % 64.  Rows >= M were staged from zero accumulators.
+    // qkv bias gradient folded in: column sums of the three staged [128 x HD] tiles (the bf16 values that are stored), one
+    // atomicAdd per column per CTA -- replaces a separate pass over dqkv (18 us per layer).  hd 64: thread t: tile t / 64 (and
+    // the third tile split by halves), column t % 64; hd 128: column t of all three tiles.  Rows >= M were staged from zero
+    // accumulators.
     const int c = tid & 63, chunk = c >> 3, within = (c & 7) * 2;
     auto colsum_rows = [&](const uint8_t* tile, int r0, int r1) {
       float acc = 0.f;
@@ -1037,21 +1087,29 @@ __global__ void __launch_bounds__(128, 2) attn_bwd_small_kernel(const __grid_con
         acc += __bfloat162float(*reinterpret_cast<const __nv_bfloat16*>(tile + r * 128 + ((chunk ^ (r & 7)) << 4) + within));
       return acc;
     };
-    const int t01 = tid >> 6;  // 0: dQ tile, 1: dK tile
-    atomicAdd(p.dbias + (t01 == 0 ? colQ : colK) + c, colsum_rows(smem + t01 * kTile, 0, kBlk));
-    atomicAdd(p.dbias + colV + c, colsum_rows(smem + 2 * kTile, t01 * 64, t01 * 64 + 64));
+    if constexpr (HD == 64) {
+      const int t01 = tid >> 6;  // 0: dQ tile, 1: dK tile
+      atomicAdd(p.dbias + (t01 == 0 ? colQ : colK) + c, colsum_rows(smem + t01 * kTile, 0, kBlk));
+      atomicAdd(p.dbias + colV + c, colsum_rows(smem + 2 * kTile, t01 * 64, t01 * 64 + 64));
+    } else {
+      const int atom = tid >> 6;  // column tid = atom tid / 64, column tid % 64 inside it
+#pragma unroll 1
+      for (int which = 0; which < 3; ++which)
+        atomicAdd(p.dbias + (which == 0 ? colQ : (which == 1 ? colK : colV)) + tid,
+                  colsum_rows(smem + which * kOp + atom * kTile, 0, kBlk));
+    }
   }
   if (warp == 0) {
     if (elect_one()) {
-      tma_store_2d(&p.tmap_out, smem, colQ, q0);
-      tma_store_2d(&p.tmap_out, smem + kTile, colK, q0);
-      tma_store_2d(&p.tmap_out, smem + 2 * kTile, colV, q0);
+      tma_store_tile<HD>(&p.tmap_out, smem, colQ, q0);
+      tma_store_tile<HD>(&p.tmap_out, smem + kOp, colK, q0);
+      tma_store_tile<HD>(&p.tmap_out, smem + 2 * kOp, colV, q0);
       tma_store_commit();
       tma_store_wait_read<0>();
     }
     __syncwarp();
     tc_fence_after();
-    tmem_dealloc(tmem, 256);
+    tmem_dealloc(tmem, kCols);
   }
 }
 
@@ -1066,63 +1124,79 @@ static void set_drop(AttnParams& p, const void* rng, int stream, float prob) {
   p.drop.scale = 1.f / (1.f - prob);
 }
 
-extern "C" int dtb_attention_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, int Hkv, int hd, int ld_qkv,
-                                 int ld_out, float scale, cudaStream_t s, const void* rng, int drop_stream, float drop_p,
-                                 const int* kv_len) {
-  if (hd != kHd || H % Hkv != 0) return 10;
-  AttnParams p{};
-  p.kv_len = kv_len;
-  set_drop(p, rng, drop_stream, drop_p);
+template <int HD>
+static int attention_fwd_hd(AttnParams& p, const void* qkv, void* out, int B, int T, int H, int Hkv, int ld_qkv, int ld_out,
+                            cudaStream_t s) {
   const int M = B * T;
-  if (make_tmap_2d(&p.tmap_qkv, qkv, 2, uint64_t(H + 2 * Hkv) * kHd, M, ld_qkv, 64, kBlk)) return 11;
+  if (make_tmap_2d(&p.tmap_qkv, qkv, 2, uint64_t(H + 2 * Hkv) * HD, M, ld_qkv, 64, kBlk)) return 11;
   p.tmap_do = p.tmap_qkv;
-  if (make_tmap_2d(&p.tmap_out, out, 2, uint64_t(H) * kHd, M, ld_out, 64, kBlk)) return 11;
-  p.out = (__nv_bfloat16*)out; p.lse = lse; p.M = M; p.T = T; p.H = H; p.Hkv = Hkv; p.ld_out = ld_out; p.ld_o = ld_out;
-  p.scale = scale;
+  if (make_tmap_2d(&p.tmap_out, out, 2, uint64_t(H) * HD, M, ld_out, 64, kBlk)) return 11;
   static bool cfg = false;
   if (!cfg) {
-    if (cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdSmem) != cudaSuccess) return 12;
-    if (cudaFuncSetAttribute(attn_fwd_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdSmallSmem) != cudaSuccess) return 12;
+    if (cudaFuncSetAttribute(attn_fwd_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<HD>()) != cudaSuccess) return 12;
+    if (cudaFuncSetAttribute(attn_fwd_small_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_small_smem<HD>()) != cudaSuccess)
+      return 12;
     cfg = true;
   }
   dim3 grid((M + kBlk - 1) / kBlk, H);
   static const bool no_small = getenv("DTB200_ATTN_NO_SMALL") != nullptr;
-  if (kBlk % T == 0 && !no_small) launch_pdl(attn_fwd_small_kernel, grid, dim3(128), kFwdSmallSmem, s, p);  // self-contained blocks
-  else attn_fwd_kernel<<<grid, 128, kFwdSmem, s>>>(p);
+  if (kBlk % T == 0 && !no_small) launch_pdl(attn_fwd_small_kernel<HD>, grid, dim3(128), fwd_small_smem<HD>(), s, p);  // self-contained blocks
+  else attn_fwd_kernel<HD><<<grid, 128, fwd_smem<HD>(), s>>>(p);
+  return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+
+extern "C" int dtb_attention_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, int Hkv, int hd, int ld_qkv,
+                                 int ld_out, float scale, cudaStream_t s, const void* rng, int drop_stream, float drop_p,
+                                 const int* kv_len) {
+  if ((hd != 64 && hd != 128) || H % Hkv != 0) return 10;
+  AttnParams p{};
+  p.kv_len = kv_len;
+  set_drop(p, rng, drop_stream, drop_p);
+  p.out = (__nv_bfloat16*)out; p.lse = lse; p.M = B * T; p.T = T; p.H = H; p.Hkv = Hkv; p.ld_out = ld_out; p.ld_o = ld_out;
+  p.scale = scale;
+  return hd == 64 ? attention_fwd_hd<64>(p, qkv, out, B, T, H, Hkv, ld_qkv, ld_out, s)
+                  : attention_fwd_hd<128>(p, qkv, out, B, T, H, Hkv, ld_qkv, ld_out, s);
+}
+
+template <int HD>
+static int attention_bwd_hd(AttnParams& p, const void* dout, const void* qkv, const void* o, void* dqkv, int B, int T, int H,
+                            int Hkv, int ld_qkv, int ld_o, cudaStream_t s) {
+  const int M = B * T;
+  if (make_tmap_2d(&p.tmap_qkv, qkv, 2, uint64_t(H + 2 * Hkv) * HD, M, ld_qkv, 64, kBlk)) return 11;
+  if (make_tmap_2d(&p.tmap_do, dout, 2, uint64_t(H) * HD, M, ld_o, 64, kBlk)) return 11;
+  if (make_tmap_2d(&p.tmap_o, o, 2, uint64_t(H) * HD, M, ld_o, 64, kBlk)) return 11;
+  if (make_tmap_2d(&p.tmap_out, dqkv, 2, uint64_t(H + 2 * Hkv) * HD, M, ld_qkv, 64, kBlk)) return 11;
+  static bool cfg = false;
+  if (!cfg) {
+    if (cudaFuncSetAttribute(attn_bwd_kv_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd_kv_smem<HD>()) != cudaSuccess) return 12;
+    if (cudaFuncSetAttribute(attn_bwd_q_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd_q_smem<HD>()) != cudaSuccess) return 12;
+    if (cudaFuncSetAttribute(attn_bwd_small_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd_small_smem<HD>()) != cudaSuccess)
+      return 12;
+    cfg = true;
+  }
+  const int nblk = (M + kBlk - 1) / kBlk;
+  static const bool no_small = getenv("DTB200_ATTN_NO_SMALL") != nullptr;
+  if (p.dbias && !(kBlk % T == 0 && H == Hkv && !no_small)) return 13;  // the fold exists in the single-block kernel only
+  if (kBlk % T == 0 && H == Hkv && !no_small) {
+    launch_pdl(attn_bwd_small_kernel<HD>, dim3(nblk, H), dim3(128), bwd_small_smem<HD>(), s, p);
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+  }
+  attn_bwd_kv_kernel<HD><<<dim3(nblk, Hkv), 128, bwd_kv_smem<HD>(), s>>>(p);
+  if (cudaGetLastError() != cudaSuccess) return 1;
+  attn_bwd_q_kernel<HD><<<dim3(nblk, H), 128, bwd_q_smem<HD>(), s>>>(p);
   return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
 extern "C" int dtb_attention_bwd(const void* dout, const void* qkv, const void* o, const float* lse, void* dqkv, int B, int T,
                                  int H, int Hkv, int hd, int ld_qkv, int ld_o, float scale, cudaStream_t s, const void* rng,
                                  int drop_stream, float drop_p, float* dbias, const int* kv_len) {
-  if (hd != kHd || H % Hkv != 0) return 10;
+  if ((hd != 64 && hd != 128) || H % Hkv != 0) return 10;
   AttnParams p{};
   p.dbias = dbias;
   p.kv_len = kv_len;
   set_drop(p, rng, drop_stream, drop_p);
-  const int M = B * T;
-  if (make_tmap_2d(&p.tmap_qkv, qkv, 2, uint64_t(H + 2 * Hkv) * kHd, M, ld_qkv, 64, kBlk)) return 11;
-  if (make_tmap_2d(&p.tmap_do, dout, 2, uint64_t(H) * kHd, M, ld_o, 64, kBlk)) return 11;
-  if (make_tmap_2d(&p.tmap_o, o, 2, uint64_t(H) * kHd, M, ld_o, 64, kBlk)) return 11;
-  if (make_tmap_2d(&p.tmap_out, dqkv, 2, uint64_t(H + 2 * Hkv) * kHd, M, ld_qkv, 64, kBlk)) return 11;
   p.o = (const __nv_bfloat16*)o; p.dout = (const __nv_bfloat16*)dout; p.out = (__nv_bfloat16*)dqkv;
-  p.lse = const_cast<float*>(lse); p.M = M; p.T = T; p.H = H; p.Hkv = Hkv; p.ld_out = ld_qkv; p.ld_o = ld_o; p.scale = scale;
-  static bool cfg = false;
-  if (!cfg) {
-    if (cudaFuncSetAttribute(attn_bwd_kv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBwdKvSmem) != cudaSuccess) return 12;
-    if (cudaFuncSetAttribute(attn_bwd_q_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBwdQSmem) != cudaSuccess) return 12;
-    if (cudaFuncSetAttribute(attn_bwd_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBwdSmallSmem) != cudaSuccess) return 12;
-    cfg = true;
-  }
-  const int nblk = (M + kBlk - 1) / kBlk;
-  static const bool no_small = getenv("DTB200_ATTN_NO_SMALL") != nullptr;
-  if (dbias && !(kBlk % T == 0 && H == Hkv && !no_small)) return 13;  // the fold exists in the single-block kernel only
-  if (kBlk % T == 0 && H == Hkv && !no_small) {
-    launch_pdl(attn_bwd_small_kernel, dim3(nblk, H), dim3(128), kBwdSmallSmem, s, p);
-    return cudaGetLastError() == cudaSuccess ? 0 : 1;
-  }
-  attn_bwd_kv_kernel<<<dim3(nblk, Hkv), 128, kBwdKvSmem, s>>>(p);
-  if (cudaGetLastError() != cudaSuccess) return 1;
-  attn_bwd_q_kernel<<<dim3(nblk, H), 128, kBwdQSmem, s>>>(p);
-  return cudaGetLastError() == cudaSuccess ? 0 : 1;
+  p.lse = const_cast<float*>(lse); p.M = B * T; p.T = T; p.H = H; p.Hkv = Hkv; p.ld_out = ld_qkv; p.ld_o = ld_o; p.scale = scale;
+  return hd == 64 ? attention_bwd_hd<64>(p, dout, qkv, o, dqkv, B, T, H, Hkv, ld_qkv, ld_o, s)
+                  : attention_bwd_hd<128>(p, dout, qkv, o, dqkv, B, T, H, Hkv, ld_qkv, ld_o, s);
 }

@@ -38,6 +38,10 @@ class ModelConfig:
     ffn: Optional[int] = None
     eps: float = 1e-5
     rope_theta: float = 500000.0
+    # RoPE frequency scaling as sorted (key, value) pairs (a tuple keeps the config hashable and comparable), e.g.
+    # (("factor", 32.0), ("high_freq_factor", 4.0), ("low_freq_factor", 1.0), ("original_max_position_embeddings", 8192),
+    #  ("rope_type", "llama3")); None = unscaled theta^(-2i/hd).  Only "llama3" is supported (see rope_inv_freq).
+    rope_scaling: Optional[Tuple[Tuple[str, object], ...]] = None
     name: str = "gpt2"
     # embd / attn / resid dropout probability in TRAIN mode.  HF GPT-2 ships 0.1 for all three and the reference miner
     # trains with it on (reference hivetrain/training_manager.py:46 ``model.train()``); Llama configs use 0.
@@ -67,6 +71,9 @@ PRESETS: Dict[str, ModelConfig] = {
     "gpt2-tiny": ModelConfig(name="gpt2-tiny", vocab_size=512, n_positions=128, n_embd=128, n_layer=2, n_head=2),
     "llama-3.2-1b": ModelConfig(family="llama", name="llama-3.2-1b", vocab_size=128256, n_positions=131072, n_embd=2048,
                                 n_layer=16, n_head=32, n_kv_head=8, ffn=8192, eps=1e-5, rope_theta=500000.0),
+    # shape preset of Llama-3.2-3B (head_dim 128); its "llama3" RoPE scaling comes from config.json on import
+    "llama-3.2-3b": ModelConfig(family="llama", name="llama-3.2-3b", vocab_size=128256, n_positions=131072, n_embd=3072,
+                                n_layer=28, n_head=24, n_kv_head=8, ffn=8192, eps=1e-5, rope_theta=500000.0),
     "llama-tiny": ModelConfig(family="llama", name="llama-tiny", vocab_size=512, n_positions=256, n_embd=128, n_layer=2,
                               n_head=4, n_kv_head=2, ffn=256, eps=1e-5, rope_theta=10000.0),
 }
@@ -190,10 +197,32 @@ def _norm(cfg, x, w, b):
     return x * rs * w
 
 
-def _rope(x, theta):  # x [B,T,h,hd]
+def rope_inv_freq(cfg: ModelConfig, device=None) -> torch.Tensor:
+    """fp32 [hd/2] RoPE inverse frequencies: theta^(-2i/hd), with ``cfg.rope_scaling`` applied.  "llama3" (Llama 3.1 / 3.2)
+    is HF's rule (``transformers.modeling_rope_utils._compute_llama3_parameters``): wavelengths longer than
+    original_max_position_embeddings / low_freq_factor are divided by ``factor``, shorter than .. / high_freq_factor kept,
+    and the band in between interpolated; the attention scale is unchanged."""
+    half = cfg.head_dim // 2
+    inv = 1.0 / (cfg.rope_theta ** (torch.arange(0, half, device=device, dtype=torch.float32) / half))
+    if cfg.rope_scaling is None:
+        return inv
+    sc = dict(cfg.rope_scaling)
+    if sc.get("rope_type") != "llama3":
+        raise ValueError(f"unsupported rope_type {sc.get('rope_type')!r}")
+    factor, lo, hi = float(sc["factor"]), float(sc["low_freq_factor"]), float(sc["high_freq_factor"])
+    old_ctx = float(sc["original_max_position_embeddings"])
+    low_wavelen, high_wavelen = old_ctx / lo, old_ctx / hi
+    wavelen = 2 * math.pi / inv
+    inv_l = torch.where(wavelen > low_wavelen, inv / factor, inv)
+    smooth = (old_ctx / wavelen - lo) / (hi - lo)
+    smoothed = (1 - smooth) * inv_l / factor + smooth * inv_l
+    medium = ~(wavelen < high_wavelen) * ~(wavelen > low_wavelen)
+    return torch.where(medium, smoothed, inv_l)
+
+
+def _rope(x, inv):  # x [B,T,h,hd], inv [hd/2] (rope_inv_freq)
     B, T, h, hd = x.shape
     half = hd // 2
-    inv = 1.0 / (theta ** (torch.arange(0, half, device=x.device, dtype=torch.float32) / half))
     ang = torch.arange(T, device=x.device, dtype=torch.float32)[:, None] * inv[None, :]
     c, s = ang.cos()[None, :, None, :], ang.sin()[None, :, None, :]
     x1, x2 = x[..., :half], x[..., half:]
@@ -242,13 +271,14 @@ def oracle_logits(cfg: ModelConfig, man: Manifest, theta: torch.Tensor, input_id
     if pd > 0:
         x = x * dm("embd")
     mask = ref.attn_mask(B, T, theta.device, kv_len_of(attention_mask, T))
+    inv_freq = rope_inv_freq(cfg, theta.device) if cfg.family == "llama" else None
     for l, L in enumerate(P.layers):
         h = _norm(cfg, x, L.ln1_w, L.ln1_b)
         qkv = F.linear(h, L.qkv_w, L.qkv_b)
         q, k, v = qkv.split([H * hd, Hkv * hd, Hkv * hd], dim=-1)
         q, k, v = q.view(B, T, H, hd), k.view(B, T, Hkv, hd), v.view(B, T, Hkv, hd)
         if cfg.family == "llama":
-            q, k = _rope(q, cfg.rope_theta), _rope(k, cfg.rope_theta)
+            q, k = _rope(q, inv_freq), _rope(k, inv_freq)
         q, k, v = q.transpose(1, 2), k.transpose(1, 2), v.transpose(1, 2)
         if Hkv != H:
             k = k.repeat_interleave(H // Hkv, dim=1)
@@ -343,6 +373,9 @@ class TransformerEngine:
         self.logits = mk(self.lm_chunk, self.ldl)
         self.losses = mk(M, dtype=f32)
         self.loss = torch.zeros((), dtype=f32, device=self.dev)
+        # scaled RoPE: the inverse-frequency table is built once here (the step stays capturable); unscaled configs pass no
+        # table and the kernel computes theta^(-2i/hd) inline
+        self.rope_inv = rope_inv_freq(cfg, self.dev) if glu and cfg.rope_scaling is not None else None
         # backward scratch
         if not self.eval_only:
             self.dx = mk(M, d)
@@ -569,7 +602,7 @@ class TransformerEngine:
             self._norm_fwd(x, Lp.ln1_w, Lp.ln1_b, self.h1[l], self.mean1[l], self.rstd1[l])
             self._fgemm(l, "qkv_w", self.h1[l], self.qkv[l], epi="bias" if Lp.qkv_b is not None else "none", bias=Lp.qkv_b)
             if cfg.family == "llama":
-                ops.rope_(self.qkv[l], B, T, H, Hkv, hd, cfg.rope_theta)
+                ops.rope_(self.qkv[l], B, T, H, Hkv, hd, cfg.rope_theta, inv_freq=self.rope_inv)
             ops.attention_fwd(self.qkv[l], self.att[l], self.lse[l], B, T, H, hd, Hkv, drop=self._drop("attn", l),
                               kv_len=self.kvlen)
             self._fgemm(l, "o_w", self.att[l], self.xmid[l], epi="bias_resid" if Lp.o_b is not None else "resid", bias=Lp.o_b,
@@ -670,7 +703,7 @@ class TransformerEngine:
             ops.attention_bwd(self.datt, self.qkv[l], self.att[l], self.lse[l], self.dqkv, B, T, H, hd, Hkv,
                               drop=self._drop("attn", l), dbias=Lg.qkv_b, kv_len=self.kvlen)
             if cfg.family == "llama":
-                ops.rope_(self.dqkv, B, T, H, Hkv, hd, cfg.rope_theta, inverse=True)
+                ops.rope_(self.dqkv, B, T, H, Hkv, hd, cfg.rope_theta, inverse=True, inv_freq=self.rope_inv)
             self._dgemm(l, "qkv_w", self.dqkv, self.dh)
             ops.gemm(self.dqkv, self.h1[l], Lg.qkv_w, a_mn=True, b_mn=True, accumulate=True)
             nxt = l - 1
@@ -756,8 +789,36 @@ def pack_any(man: Manifest, blob, cfg: Optional[ModelConfig] = None) -> torch.Te
     return man.pack(blob, torch.zeros(man.total, dtype=torch.float32))
 
 
+def _rope_from_hf(d: dict) -> Tuple[float, Optional[Tuple[Tuple[str, object], ...]]]:
+    """(theta, scaling) of an HF Llama config in either layout: top-level ``rope_theta`` / ``rope_scaling`` (transformers 4)
+    or ``rope_parameters`` (transformers >= 5).  No type or "default" = unscaled; "llama3" is kept; anything else raises."""
+    rp = d.get("rope_parameters") or {}
+    theta = float(rp.get("rope_theta", d.get("rope_theta", 10000.0)))
+    sc = d.get("rope_scaling") or (rp if "rope_type" in rp or "type" in rp else None)
+    if not sc:
+        return theta, None
+    rt = sc.get("rope_type", sc.get("type", "default"))
+    if rt == "default":
+        return theta, None
+    if rt != "llama3":
+        raise ValueError(f"unsupported RoPE scaling type {rt!r} (supported: default, llama3)")
+    keep = ("factor", "low_freq_factor", "high_freq_factor", "original_max_position_embeddings")
+    missing = [k for k in keep if k not in sc]
+    if missing:
+        raise ValueError(f"llama3 RoPE scaling lacks {missing}")
+    vals = {k: float(sc[k]) for k in keep}
+    vals["original_max_position_embeddings"] = int(sc["original_max_position_embeddings"])
+    vals["rope_type"] = "llama3"
+    return theta, tuple(sorted(vals.items()))
+
+
 def config_from_hf(d: dict) -> ModelConfig:
-    """``config.json`` of an HF GPT-2 / Llama checkpoint -> ModelConfig."""
+    """``config.json`` of an HF GPT-2 / Llama checkpoint -> ModelConfig.
+
+    Llama: RoPE theta and "llama3" scaling are read from either config layout (:func:`_rope_from_hf`); ``head_dim``, when
+    present, must equal hidden_size / num_attention_heads; the LM head must be tied to the embedding
+    (``tie_word_embeddings``, False when absent as in ``transformers.LlamaConfig``) -- an untied head has no place in the
+    arena, and loading it as tied would silently be a different model."""
     mt = d.get("model_type", "gpt2")
     if mt == "gpt2":
         return ModelConfig(family="gpt2", name=d.get("_name_or_path") or "gpt2-hf", vocab_size=int(d["vocab_size"]),
@@ -765,12 +826,19 @@ def config_from_hf(d: dict) -> ModelConfig:
                            n_head=int(d["n_head"]), ffn=d.get("n_inner") or None, eps=float(d.get("layer_norm_epsilon", 1e-5)),
                            dropout=float(d.get("resid_pdrop", 0.1)))
     if mt == "llama":
+        d_model, n_head = int(d["hidden_size"]), int(d["num_attention_heads"])
+        if d.get("head_dim") is not None and int(d["head_dim"]) * n_head != d_model:
+            raise ValueError(f"head_dim {d['head_dim']} != hidden_size / num_attention_heads = {d_model} / {n_head}: "
+                             "a decoupled head dim is not supported")
+        if not d.get("tie_word_embeddings", False):
+            raise ValueError("tie_word_embeddings is false: an untied LM head is not supported")
+        theta, scaling = _rope_from_hf(d)
         return ModelConfig(family="llama", name=d.get("_name_or_path") or "llama-hf", vocab_size=int(d["vocab_size"]),
-                           n_positions=int(d.get("max_position_embeddings", 8192)), n_embd=int(d["hidden_size"]),
-                           n_layer=int(d["num_hidden_layers"]), n_head=int(d["num_attention_heads"]),
-                           n_kv_head=int(d.get("num_key_value_heads", d["num_attention_heads"])),
+                           n_positions=int(d.get("max_position_embeddings", 8192)), n_embd=d_model,
+                           n_layer=int(d["num_hidden_layers"]), n_head=n_head,
+                           n_kv_head=int(d.get("num_key_value_heads") or n_head),
                            ffn=int(d["intermediate_size"]), eps=float(d.get("rms_norm_eps", 1e-5)),
-                           rope_theta=float(d.get("rope_theta", 10000.0)))
+                           rope_theta=theta, rope_scaling=scaling)
     raise ValueError(f"unsupported HF model_type {mt!r}")
 
 

@@ -302,11 +302,13 @@ def swiglu_bwd(dout, gu, dgu):
     return dgu
 
 
-def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False):
+def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False, inv_freq=None):
+    """``inv_freq`` (fp32 [hd/2] on the device, optional): precomputed inverse frequencies (``models.transformer.rope_inv_freq``
+    of a scaled config); None = ``theta ** (-2i/hd)`` computed inline."""
     if not use_kernels(qkv):
-        return ref.rope_(qkv, B, T, H, Hkv, hd, theta, inverse)
+        return ref.rope_(qkv, B, T, H, Hkv, hd, theta, inverse, inv_freq)
     _c(_lib.lib().dtb_rope(_lib.ptr(qkv), B * T, T, H + Hkv, qkv.shape[1], hd, ctypes.c_float(theta), int(inverse),
-                           _lib.num_sms(), _lib.stream_ptr()), "rope")
+                           _lib.num_sms(), _lib.stream_ptr(), _lib.ptr(inv_freq)), "rope")
     _tick()
     return qkv
 

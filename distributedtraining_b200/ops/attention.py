@@ -15,7 +15,7 @@ def _kernel_ok(qkv, T, hd) -> bool:
     if not _lib.use_kernels(qkv):
         return False
     L = _lib.lib()
-    return hasattr(L, "dtb_attention_fwd") and hd == 64
+    return hasattr(L, "dtb_attention_fwd") and hd in (64, 128)
 
 
 def attention_fwd(qkv, out, lse, B, T, H, hd, Hkv=None, drop=None, kv_len=None):

@@ -271,11 +271,15 @@ def attention_bwd(dout, qkv, out, lse, dqkv, B, T, H, hd, Hkv=None, drop=None, k
     return dqkv
 
 
-def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False):
-    """In-place rotary embedding (rotate-half convention) on the q and k parts of packed qkv."""
+def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False, inv_freq=None):
+    """In-place rotary embedding (rotate-half convention) on the q and k parts of packed qkv.  ``inv_freq`` (fp32 [hd/2],
+    optional) replaces the unscaled ``theta ** (-2i/hd)`` frequencies (see ``models.transformer.rope_inv_freq``)."""
     dev = qkv.device
     half = hd // 2
-    inv = 1.0 / (theta ** (torch.arange(0, half, device=dev, dtype=torch.float32) / half))
+    if inv_freq is not None:
+        inv = inv_freq.to(device=dev, dtype=torch.float32)
+    else:
+        inv = 1.0 / (theta ** (torch.arange(0, half, device=dev, dtype=torch.float32) / half))
     ang = torch.arange(T, device=dev, dtype=torch.float32)[:, None] * inv[None, :]
     cos, sin = ang.cos(), ang.sin()
     if inverse:
