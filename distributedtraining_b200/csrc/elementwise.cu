@@ -1,9 +1,11 @@
 // Bandwidth-bound transformer kernels for sm_100a: embedding fwd/bwd, LayerNorm / RMSNorm fwd+bwd, fused
-// cross-entropy (loss + dlogits in place, row resident in shared memory), column sums (bias grads), SwiGLU, RoPE.
+// cross-entropy (loss + dlogits in place, row resident in shared memory), column sums (bias grads), SwiGLU, RoPE, and
+// Qwen3's fused QK-norm + RoPE.
 // All of them are single-pass, 128-bit vectorised, fp32 math on bf16 storage.
 //
 // Parity: these replace the ATen kernels behind HF GPT-2 in the reference miner/validator/averager hot loops
 // (reference hivetrain/training_manager.py:380-392; SURVEY.md K1, K2, K8, K9).
+#include <algorithm>
 #include <cstdint>
 #include <cstdlib>
 #include <cuda_bf16.h>
@@ -750,6 +752,156 @@ __global__ void rope_kernel(bf16* __restrict__ qkv, int M, int T, int nheads_rot
   }
 }
 
+// Qwen3 QK-norm + RoPE, fused and in place on the q|k heads of packed qkv [M, ld] (ld >= (H+2Hkv)*HD): per-head RMSNorm
+// (q_norm weights for heads < H, k_norm for the Hkv k heads; fp32 statistics), then rotate-half RoPE by (row % T) * inv_freq[p],
+// rounded once to bf16.  One warp per (row, q-or-k head); lane l holds the PPL = HD/64 pairs p = l*PPL.. and their rotate-half
+// partners p + HD/2, so the rotation needs no shuffles and the norm sum is one warp reduction.  v is not touched.
+template <int N>
+__device__ __forceinline__ void ld_bf(const bf16* p, float* f) {
+  if constexpr (N == 2) {
+    const float2 t = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(p));
+    f[0] = t.x;
+    f[1] = t.y;
+  } else {
+    f[0] = __bfloat162float(*p);
+  }
+}
+template <int N>
+__device__ __forceinline__ void st_bf(bf16* p, const float* f) {
+  if constexpr (N == 2) *reinterpret_cast<__nv_bfloat162*>(p) = __floats2bfloat162_rn(f[0], f[1]);
+  else *p = __float2bfloat16(f[0]);
+}
+
+// Forward.  raw / rstd_out (optional, both or neither): the q|k input [M, nh*HD] bf16 and the per-head rstd [M, nh] fp32
+// that the backward needs.
+template <int HD>
+__global__ void __launch_bounds__(256) qk_norm_rope_fwd_kernel(bf16* __restrict__ qkv, int ld, int M, int T, int H, int nh,
+                                                               const bf16* __restrict__ qw, const bf16* __restrict__ kw,
+                                                               float eps, const float* __restrict__ inv_freq,
+                                                               bf16* __restrict__ raw, float* __restrict__ rstd_out) {
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent kernel may start its prologue (sm100_ptx.cuh)
+  constexpr int HALF = HD / 2, PPL = HD / 64;
+  const int lane = threadIdx.x & 31;
+  const int p0 = lane * PPL;
+  float inv[PPL], wq[2 * PPL], wk[2 * PPL];
+  ld_bf<PPL>(qw + p0, wq);
+  ld_bf<PPL>(qw + HALF + p0, wq + PPL);
+  ld_bf<PPL>(kw + p0, wk);
+  ld_bf<PPL>(kw + HALF + p0, wk + PPL);
+#pragma unroll
+  for (int k = 0; k < PPL; ++k) inv[k] = __ldg(inv_freq + p0 + k);
+  const size_t items = size_t(M) * nh;
+  const size_t nwarps = (size_t(gridDim.x) * blockDim.x) >> 5;
+  for (size_t it = (size_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; it < items; it += nwarps) {
+    const int h = int(it % nh);
+    const size_t row = it / nh;
+    const float t = float(int(row % T));
+    bf16* base = qkv + row * ld + size_t(h) * HD;
+    float a[PPL], b[PPL];
+    ld_bf<PPL>(base + p0, a);
+    ld_bf<PPL>(base + HALF + p0, b);
+    if (raw) {
+      st_bf<PPL>(raw + it * HD + p0, a);
+      st_bf<PPL>(raw + it * HD + HALF + p0, b);
+    }
+    float ss = 0.f;
+#pragma unroll
+    for (int k = 0; k < PPL; ++k) ss += a[k] * a[k] + b[k] * b[k];
+    const float rs = rsqrtf(warp_sum(ss) * (1.f / HD) + eps);
+    if (rstd_out && lane == 0) rstd_out[it] = rs;
+    const bool is_q = h < H;
+#pragma unroll
+    for (int k = 0; k < PPL; ++k) {
+      const float ya = a[k] * rs * (is_q ? wq[k] : wk[k]), yb = b[k] * rs * (is_q ? wq[PPL + k] : wk[PPL + k]);
+      float s, c;
+      sincosf(t * inv[k], &s, &c);
+      a[k] = ya * c - yb * s;
+      b[k] = yb * c + ya * s;
+    }
+    st_bf<PPL>(base + p0, a);
+    st_bf<PPL>(base + HALF + p0, b);
+  }
+}
+
+// Backward, in place on the q|k heads of dqkv: g = R(-theta) dy, x^ = raw * rstd, dx = rstd * (g w - x^ mean(g w x^)).
+// dw += sum g x^: per-lane register partials (q and k apart), reduced per CTA in shared memory, then ONE fp32 atomicAdd per
+// element per CTA into dqw / dkw (as norm_bwd_kernel does).
+template <int HD>
+__global__ void __launch_bounds__(256) qk_norm_rope_bwd_kernel(bf16* __restrict__ dqkv, int ld, int M, int T, int H, int nh,
+                                                               const bf16* __restrict__ qw, const bf16* __restrict__ kw,
+                                                               const float* __restrict__ inv_freq, const bf16* __restrict__ raw,
+                                                               const float* __restrict__ rstd, float* __restrict__ dqw,
+                                                               float* __restrict__ dkw) {
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // PDL: a dependent kernel may start its prologue (sm100_ptx.cuh)
+  constexpr int HALF = HD / 2, PPL = HD / 64;
+  __shared__ float s_dw[2 * HD];  // [q | k]
+  for (int i = threadIdx.x; i < 2 * HD; i += blockDim.x) s_dw[i] = 0.f;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int p0 = lane * PPL;
+  float inv[PPL], wq[2 * PPL], wk[2 * PPL], aq[2 * PPL], ak[2 * PPL];
+  ld_bf<PPL>(qw + p0, wq);
+  ld_bf<PPL>(qw + HALF + p0, wq + PPL);
+  ld_bf<PPL>(kw + p0, wk);
+  ld_bf<PPL>(kw + HALF + p0, wk + PPL);
+#pragma unroll
+  for (int k = 0; k < PPL; ++k) inv[k] = __ldg(inv_freq + p0 + k);
+#pragma unroll
+  for (int k = 0; k < 2 * PPL; ++k) aq[k] = ak[k] = 0.f;
+  const size_t items = size_t(M) * nh;
+  const size_t nwarps = (size_t(gridDim.x) * blockDim.x) >> 5;
+  for (size_t it = (size_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; it < items; it += nwarps) {
+    const int h = int(it % nh);
+    const size_t row = it / nh;
+    const float t = float(int(row % T));
+    bf16* base = dqkv + row * ld + size_t(h) * HD;
+    float da[PPL], db[PPL], xa[PPL], xb[PPL];
+    ld_bf<PPL>(base + p0, da);
+    ld_bf<PPL>(base + HALF + p0, db);
+    ld_bf<PPL>(raw + it * HD + p0, xa);
+    ld_bf<PPL>(raw + it * HD + HALF + p0, xb);
+    const float rs = __ldg(rstd + it);
+    const bool is_q = h < H;
+    float ga[PPL], gb[PPL], wa[PPL], wb[PPL], dot = 0.f;
+#pragma unroll
+    for (int k = 0; k < PPL; ++k) {
+      float s, c;
+      sincosf(t * inv[k], &s, &c);
+      ga[k] = da[k] * c + db[k] * s;
+      gb[k] = db[k] * c - da[k] * s;
+      xa[k] *= rs;
+      xb[k] *= rs;
+      wa[k] = is_q ? wq[k] : wk[k];
+      wb[k] = is_q ? wq[PPL + k] : wk[PPL + k];
+      dot += ga[k] * wa[k] * xa[k] + gb[k] * wb[k] * xb[k];
+      if (is_q) {
+        aq[k] += ga[k] * xa[k];
+        aq[PPL + k] += gb[k] * xb[k];
+      } else {
+        ak[k] += ga[k] * xa[k];
+        ak[PPL + k] += gb[k] * xb[k];
+      }
+    }
+    dot = warp_sum(dot) * (1.f / HD);
+#pragma unroll
+    for (int k = 0; k < PPL; ++k) {
+      da[k] = rs * (ga[k] * wa[k] - xa[k] * dot);
+      db[k] = rs * (gb[k] * wb[k] - xb[k] * dot);
+    }
+    st_bf<PPL>(base + p0, da);
+    st_bf<PPL>(base + HALF + p0, db);
+  }
+#pragma unroll
+  for (int k = 0; k < PPL; ++k) {
+    atomicAdd(&s_dw[p0 + k], aq[k]);
+    atomicAdd(&s_dw[HALF + p0 + k], aq[PPL + k]);
+    atomicAdd(&s_dw[HD + p0 + k], ak[k]);
+    atomicAdd(&s_dw[HD + HALF + p0 + k], ak[PPL + k]);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 2 * HD; i += blockDim.x) atomicAdd(i < HD ? dqw + i : dkw + (i - HD), s_dw[i]);
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // fp8 (e4m3) per-tensor quantisation with DELAYED scaling: q = sat(x / scale_in); amax_out = max|x| (for the next step)
 // ------------------------------------------------------------------------------------------------------------------
@@ -973,6 +1125,45 @@ extern "C" int dtb_rope(void* qkv, int M, int T, int nheads_rot, int row_stride,
                         cudaStream_t s, const float* inv_freq) {
   rope_kernel<<<num_sms * 8, 256, 0, s>>>((bf16*)qkv, M, T, nheads_rot, row_stride, hd, log2f(theta), inverse ? -1.f : 1.f,
                                           inv_freq);
+  return KCHECK();
+}
+// Qwen3 QK-norm + RoPE.  Errors: 1 = head dim other than 64 / 128, 2 = row stride or base pointer not aligned for the
+// 2-element accesses of hd 128 (or stride shorter than the packed row), 3 = only one of raw / rstd given.
+static int qk_norm_check(const void* qkv, int ld, int H, int Hkv, int hd) {
+  if (hd != 64 && hd != 128) return 1;
+  if (ld < (H + 2 * Hkv) * hd || (hd == 128 && (ld % 2 != 0 || reinterpret_cast<uintptr_t>(qkv) % 4 != 0))) return 2;
+  return 0;
+}
+static int qk_norm_grid(size_t items, int cap) { return int(std::min<size_t>((items + 7) / 8, size_t(cap))); }
+extern "C" int dtb_qk_norm_rope_fwd(void* qkv, int ld, int M, int T, int H, int Hkv, int hd, const void* qw, const void* kw, float eps,
+                                    const float* inv_freq, void* raw, float* rstd, int num_sms, cudaStream_t s) {
+  if (const int rc = qk_norm_check(qkv, ld, H, Hkv, hd)) return rc;
+  if ((raw == nullptr) != (rstd == nullptr)) return 3;
+  const size_t items = size_t(M) * (H + Hkv);
+  if (items == 0) return 0;
+  const int grid = qk_norm_grid(items, num_sms * 8);
+  if (hd == 128)
+    qk_norm_rope_fwd_kernel<128><<<grid, 256, 0, s>>>((bf16*)qkv, ld, M, T, H, H + Hkv, (const bf16*)qw, (const bf16*)kw, eps,
+                                                      inv_freq, (bf16*)raw, rstd);
+  else
+    qk_norm_rope_fwd_kernel<64><<<grid, 256, 0, s>>>((bf16*)qkv, ld, M, T, H, H + Hkv, (const bf16*)qw, (const bf16*)kw, eps,
+                                                     inv_freq, (bf16*)raw, rstd);
+  return KCHECK();
+}
+extern "C" int dtb_qk_norm_rope_bwd(void* dqkv, int ld, int M, int T, int H, int Hkv, int hd, const void* qw, const void* kw,
+                                    const float* inv_freq, const void* raw, const float* rstd, float* dqw, float* dkw, int num_sms,
+                                    cudaStream_t s) {
+  if (const int rc = qk_norm_check(dqkv, ld, H, Hkv, hd)) return rc;
+  if (raw == nullptr || rstd == nullptr) return 3;
+  const size_t items = size_t(M) * (H + Hkv);
+  if (items == 0) return 0;
+  const int grid = qk_norm_grid(items, num_sms * 4);  // fewer CTAs than the forward: each one flushes 2*hd global atomics
+  if (hd == 128)
+    qk_norm_rope_bwd_kernel<128><<<grid, 256, 0, s>>>((bf16*)dqkv, ld, M, T, H, H + Hkv, (const bf16*)qw, (const bf16*)kw, inv_freq,
+                                                      (const bf16*)raw, rstd, dqw, dkw);
+  else
+    qk_norm_rope_bwd_kernel<64><<<grid, 256, 0, s>>>((bf16*)dqkv, ld, M, T, H, H + Hkv, (const bf16*)qw, (const bf16*)kw, inv_freq,
+                                                     (const bf16*)raw, rstd, dqw, dkw);
   return KCHECK();
 }
 extern "C" int dtb_quant_fp8(const void* x, void* q, const float* scale_in, float* amax_out, size_t n, int num_sms, cudaStream_t s,

@@ -1,4 +1,4 @@
-"""Decoder-only transformer family (GPT-2 and Llama shapes) on flat arenas.
+"""Decoder-only transformer family (GPT-2, Llama and Qwen3 shapes) on flat arenas.
 
 Two implementations of the same maths:
 
@@ -46,10 +46,15 @@ class ModelConfig:
     # embd / attn / resid dropout probability in TRAIN mode.  HF GPT-2 ships 0.1 for all three and the reference miner
     # trains with it on (reference hivetrain/training_manager.py:46 ``model.train()``); Llama configs use 0.
     dropout: float = 0.0
+    # attention head dim when it is decoupled from the model width (Qwen3: n_head * head_dim != n_embd); None = n_embd / n_head
+    n_head_dim: Optional[int] = None
+    # Qwen3 QK-norm: an RMSNorm over every q and k head (weights [head_dim] shared across heads) between the QKV projection
+    # and RoPE (llama family only)
+    qk_norm: bool = False
 
     @property
     def head_dim(self) -> int:
-        return self.n_embd // self.n_head
+        return self.n_head_dim or self.n_embd // self.n_head
 
     @property
     def kv_heads(self) -> int:
@@ -76,6 +81,20 @@ PRESETS: Dict[str, ModelConfig] = {
                                 n_layer=28, n_head=24, n_kv_head=8, ffn=8192, eps=1e-5, rope_theta=500000.0),
     "llama-tiny": ModelConfig(family="llama", name="llama-tiny", vocab_size=512, n_positions=256, n_embd=128, n_layer=2,
                               n_head=4, n_kv_head=2, ffn=256, eps=1e-5, rope_theta=10000.0),
+    # Qwen3 dense models with a tied LM head: the Llama block plus QK-norm, head_dim 128 decoupled from the width, unscaled
+    # RoPE (theta 1e6).  Raw vocabulary; an imported checkpoint directory gets the [PAD] row on top (get_config).
+    "qwen3-0.6b": ModelConfig(family="llama", name="qwen3-0.6b", vocab_size=151936, n_positions=40960, n_embd=1024,
+                              n_layer=28, n_head=16, n_kv_head=8, n_head_dim=128, ffn=3072, eps=1e-6, rope_theta=1e6,
+                              qk_norm=True),
+    "qwen3-1.7b": ModelConfig(family="llama", name="qwen3-1.7b", vocab_size=151936, n_positions=40960, n_embd=2048,
+                              n_layer=28, n_head=16, n_kv_head=8, n_head_dim=128, ffn=6144, eps=1e-6, rope_theta=1e6,
+                              qk_norm=True),
+    "qwen3-4b": ModelConfig(family="llama", name="qwen3-4b", vocab_size=151936, n_positions=40960, n_embd=2560,
+                            n_layer=36, n_head=32, n_kv_head=8, n_head_dim=128, ffn=9728, eps=1e-6, rope_theta=1e6,
+                            qk_norm=True),
+    # test shape: 4 heads x hd 64 = 256 != n_embd 128 (decoupled head dim)
+    "qwen3-tiny": ModelConfig(family="llama", name="qwen3-tiny", vocab_size=512, n_positions=256, n_embd=128, n_layer=2,
+                              n_head=4, n_kv_head=2, n_head_dim=64, ffn=256, eps=1e-6, rope_theta=1e6, qk_norm=True),
 }
 
 
@@ -125,6 +144,10 @@ def build_manifest(cfg: ModelConfig) -> Manifest:
                 (p + "self_attn.q_proj.weight", (cfg.n_head * hd, d), "normal", True),
                 (p + "self_attn.k_proj.weight", (cfg.kv_heads * hd, d), "normal", True),
                 (p + "self_attn.v_proj.weight", (cfg.kv_heads * hd, d), "normal", True),
+            ]
+            if cfg.qk_norm:  # after v_proj: q|k|v stays one fused view, and the arena stays in program order (configure_ready)
+                e += [(p + "self_attn.q_norm.weight", (hd,), "ones", False), (p + "self_attn.k_norm.weight", (hd,), "ones", False)]
+            e += [
                 (p + "self_attn.o_proj.weight", (d, cfg.n_head * hd), "normal_resid", True),
                 (p + "post_attention_layernorm.weight", (d,), "ones", False),
                 (p + "mlp.gate_proj.weight", (Fd, d), "normal", True),
@@ -162,12 +185,15 @@ class LayerParams:
             self.ln2_w, self.ln2_b = v(p + "ln_2.weight"), v(p + "ln_2.bias")
             self.fc_w, self.fc_b = v(p + "mlp.c_fc.weight"), v(p + "mlp.c_fc.bias")
             self.proj_w, self.proj_b = v(p + "mlp.c_proj.weight"), v(p + "mlp.c_proj.bias")
+            self.q_norm = self.k_norm = None
         else:
             p = f"model.layers.{l}."
             self.ln1_w, self.ln1_b = v(p + "input_layernorm.weight"), None
             self.qkv_w = fused_view(man, flat, [p + "self_attn.q_proj.weight", p + "self_attn.k_proj.weight",
                                                 p + "self_attn.v_proj.weight"])
             self.qkv_b = None
+            self.q_norm, self.k_norm = ((v(p + "self_attn.q_norm.weight"), v(p + "self_attn.k_norm.weight")) if cfg.qk_norm
+                                        else (None, None))
             self.o_w, self.o_b = v(p + "self_attn.o_proj.weight"), None
             self.ln2_w, self.ln2_b = v(p + "post_attention_layernorm.weight"), None
             self.fc_w = fused_view(man, flat, [p + "mlp.gate_proj.weight", p + "mlp.up_proj.weight"])
@@ -277,6 +303,9 @@ def oracle_logits(cfg: ModelConfig, man: Manifest, theta: torch.Tensor, input_id
         qkv = F.linear(h, L.qkv_w, L.qkv_b)
         q, k, v = qkv.split([H * hd, Hkv * hd, Hkv * hd], dim=-1)
         q, k, v = q.view(B, T, H, hd), k.view(B, T, Hkv, hd), v.view(B, T, Hkv, hd)
+        if cfg.qk_norm:  # per-head RMSNorm before RoPE (HF Qwen3Attention)
+            q = q * torch.rsqrt(q.pow(2).mean(-1, keepdim=True) + cfg.eps) * L.q_norm
+            k = k * torch.rsqrt(k.pow(2).mean(-1, keepdim=True) + cfg.eps) * L.k_norm
         if cfg.family == "llama":
             q, k = _rope(q, inv_freq), _rope(k, inv_freq)
         q, k, v = q.transpose(1, 2), k.transpose(1, 2), v.transpose(1, 2)
@@ -374,8 +403,12 @@ class TransformerEngine:
         self.losses = mk(M, dtype=f32)
         self.loss = torch.zeros((), dtype=f32, device=self.dev)
         # scaled RoPE: the inverse-frequency table is built once here (the step stays capturable); unscaled configs pass no
-        # table and the kernel computes theta^(-2i/hd) inline
-        self.rope_inv = rope_inv_freq(cfg, self.dev) if glu and cfg.rope_scaling is not None else None
+        # table and the kernel computes theta^(-2i/hd) inline.  The fused QK-norm + RoPE kernel always reads the table.
+        self.rope_inv = rope_inv_freq(cfg, self.dev) if glu and (cfg.rope_scaling is not None or cfg.qk_norm) else None
+        # QK-norm saves for the backward: the raw q|k heads and their rstd (eval-only engines save nothing)
+        nqk = cfg.n_head + cfg.kv_heads
+        self.qk_raw = [mk(M, nqk * cfg.head_dim) for _ in range(L)] if cfg.qk_norm and not self.eval_only else None
+        self.qk_rstd = [mk(M, nqk, dtype=f32) for _ in range(L)] if cfg.qk_norm and not self.eval_only else None
         # backward scratch
         if not self.eval_only:
             self.dx = mk(M, d)
@@ -601,7 +634,10 @@ class TransformerEngine:
             x = self.xs[l]
             self._norm_fwd(x, Lp.ln1_w, Lp.ln1_b, self.h1[l], self.mean1[l], self.rstd1[l])
             self._fgemm(l, "qkv_w", self.h1[l], self.qkv[l], epi="bias" if Lp.qkv_b is not None else "none", bias=Lp.qkv_b)
-            if cfg.family == "llama":
+            if cfg.qk_norm:
+                ops.qk_norm_rope_fwd(self.qkv[l], B, T, H, Hkv, hd, Lp.q_norm, Lp.k_norm, cfg.eps, self.rope_inv,
+                                     *((self.qk_raw[l], self.qk_rstd[l]) if self.qk_raw is not None else ()))
+            elif cfg.family == "llama":
                 ops.rope_(self.qkv[l], B, T, H, Hkv, hd, cfg.rope_theta, inv_freq=self.rope_inv)
             ops.attention_fwd(self.qkv[l], self.att[l], self.lse[l], B, T, H, hd, Hkv, drop=self._drop("attn", l),
                               kv_len=self.kvlen)
@@ -702,7 +738,10 @@ class TransformerEngine:
             # d(qkv bias) = colsum(dqkv) rides on the attention backward (GPT-2 has no RoPE between the two)
             ops.attention_bwd(self.datt, self.qkv[l], self.att[l], self.lse[l], self.dqkv, B, T, H, hd, Hkv,
                               drop=self._drop("attn", l), dbias=Lg.qkv_b, kv_len=self.kvlen)
-            if cfg.family == "llama":
+            if cfg.qk_norm:
+                ops.qk_norm_rope_bwd(self.dqkv, B, T, H, Hkv, hd, Lp.q_norm, Lp.k_norm, self.rope_inv, self.qk_raw[l],
+                                     self.qk_rstd[l], Lg.q_norm, Lg.k_norm)
+            elif cfg.family == "llama":
                 ops.rope_(self.dqkv, B, T, H, Hkv, hd, cfg.rope_theta, inverse=True, inv_freq=self.rope_inv)
             self._dgemm(l, "qkv_w", self.dqkv, self.dh)
             ops.gemm(self.dqkv, self.h1[l], Lg.qkv_w, a_mn=True, b_mn=True, accumulate=True)
@@ -721,7 +760,7 @@ _CONV1D = ("c_attn.weight", "c_proj.weight", "c_fc.weight")  # HF GPT-2 stores t
 
 def to_hf_state_dict(cfg: ModelConfig, arena) -> Dict[str, torch.Tensor]:
     """HF-compatible state dict (GPT-2 Conv1D weights transposed back to [in, out]; tied lm_head added -> 149 keys):
-    loads straight into ``transformers.GPT2LMHeadModel`` / ``LlamaForCausalLM`` -- the reference's checkpoint format
+    loads straight into ``transformers.GPT2LMHeadModel`` / ``LlamaForCausalLM`` / ``Qwen3ForCausalLM`` -- the reference's checkpoint format
     (``model.state_dict()``, hivetrain/averaging_logic.py:481-488).  ``arena``: an :class:`Arena` or a flat tensor."""
     if isinstance(arena, torch.Tensor):
         arena = Arena(build_manifest(cfg), flat=arena)
@@ -746,7 +785,8 @@ def is_hf_layout(cfg: ModelConfig, sd: Dict[str, torch.Tensor]) -> bool:
 
 def from_hf_state_dict(cfg: ModelConfig, sd: Dict[str, torch.Tensor], man: Optional[Manifest] = None,
                        out: Optional[torch.Tensor] = None, resize_vocab: bool = True) -> torch.Tensor:
-    """HF state dict (``GPT2LMHeadModel`` / ``LlamaForCausalLM`` naming, or this engine's own layout) -> flat fp32 arena.
+    """HF state dict (``GPT2LMHeadModel`` / ``LlamaForCausalLM`` / ``Qwen3ForCausalLM`` naming, or this engine's own layout)
+    -> flat fp32 arena.
 
     * GPT-2 Conv1D weights are transposed to the engine's ``[out, in]`` (the square ``attn.c_proj`` cannot be told apart
       by shape -- the layout is detected on ``c_attn`` and applied to all of them);
@@ -813,12 +853,17 @@ def _rope_from_hf(d: dict) -> Tuple[float, Optional[Tuple[Tuple[str, object], ..
 
 
 def config_from_hf(d: dict) -> ModelConfig:
-    """``config.json`` of an HF GPT-2 / Llama checkpoint -> ModelConfig.
+    """``config.json`` of an HF GPT-2 / Llama / Qwen3 checkpoint -> ModelConfig.
 
     Llama: RoPE theta and "llama3" scaling are read from either config layout (:func:`_rope_from_hf`); ``head_dim``, when
     present, must equal hidden_size / num_attention_heads; the LM head must be tied to the embedding
     (``tie_word_embeddings``, False when absent as in ``transformers.LlamaConfig``) -- an untied head has no place in the
-    arena, and loading it as tied would silently be a different model."""
+    arena, and loading it as tied would silently be a different model.
+
+    Qwen3 (dense): the Llama block with QK-norm and a ``head_dim`` that may differ from hidden_size / num_attention_heads.
+    Refused with a ValueError naming the field: an untied LM head (``Qwen3Config`` defaults ``tie_word_embeddings`` to
+    False), ``attention_bias``, sliding-window attention (``use_sliding_window`` or a ``layer_types`` entry other than
+    full_attention), a ``hidden_act`` other than silu and RoPE scaling other than llama3 (YaRN)."""
     mt = d.get("model_type", "gpt2")
     if mt == "gpt2":
         return ModelConfig(family="gpt2", name=d.get("_name_or_path") or "gpt2-hf", vocab_size=int(d["vocab_size"]),
@@ -839,6 +884,26 @@ def config_from_hf(d: dict) -> ModelConfig:
                            n_kv_head=int(d.get("num_key_value_heads") or n_head),
                            ffn=int(d["intermediate_size"]), eps=float(d.get("rms_norm_eps", 1e-5)),
                            rope_theta=theta, rope_scaling=scaling)
+    if mt == "qwen3":
+        d_model, n_head = int(d["hidden_size"]), int(d["num_attention_heads"])
+        if not d.get("tie_word_embeddings", False):
+            raise ValueError("tie_word_embeddings is false: an untied LM head is not supported")
+        if d.get("attention_bias", False):
+            raise ValueError("attention_bias is true: q/k/v/o projection biases are not supported")
+        if d.get("use_sliding_window", False):
+            raise ValueError("use_sliding_window is true: sliding-window attention is not supported")
+        bad = [t for t in (d.get("layer_types") or []) if t != "full_attention"]
+        if bad:
+            raise ValueError(f"layer_types holds {sorted(set(bad))}: only full_attention layers are supported")
+        if d.get("hidden_act", "silu") != "silu":
+            raise ValueError(f"hidden_act {d['hidden_act']!r} is not supported (silu only)")
+        theta, scaling = _rope_from_hf(d)
+        return ModelConfig(family="llama", name=d.get("_name_or_path") or "qwen3-hf", vocab_size=int(d["vocab_size"]),
+                           n_positions=int(d.get("max_position_embeddings", 32768)), n_embd=d_model,
+                           n_layer=int(d["num_hidden_layers"]), n_head=n_head,
+                           n_kv_head=int(d.get("num_key_value_heads") or n_head),
+                           n_head_dim=int(d.get("head_dim") or d_model // n_head), ffn=int(d["intermediate_size"]),
+                           eps=float(d.get("rms_norm_eps", 1e-6)), rope_theta=theta, rope_scaling=scaling, qk_norm=True)
     raise ValueError(f"unsupported HF model_type {mt!r}")
 
 

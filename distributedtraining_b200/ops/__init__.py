@@ -313,6 +313,36 @@ def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False, inv_freq=None):
     return qkv
 
 
+def _qk_norm_kernel_ok(qkv, hd) -> bool:
+    return use_kernels(qkv) and hd in (64, 128)
+
+
+def qk_norm_rope_fwd(qkv, B, T, H, Hkv, hd, q_w, k_w, eps, inv_freq, raw=None, rstd=None):
+    """Qwen3 QK-norm + RoPE, in place on the q|k part of packed qkv (see :func:`reference.qk_norm_rope_fwd`).
+    ``inv_freq``: fp32 [hd/2] device table (``models.transformer.rope_inv_freq``).  ``raw`` / ``rstd``: optional saves for
+    the backward.  CUDA: one warp per (row, q-or-k head), hd 64 and 128; other head dims take the reference path."""
+    if not _qk_norm_kernel_ok(qkv, hd):
+        return ref.qk_norm_rope_fwd(qkv, B, T, H, Hkv, hd, q_w, k_w, eps, inv_freq, raw, rstd)
+    assert (raw is None) == (rstd is None)
+    _c(_lib.lib().dtb_qk_norm_rope_fwd(_lib.ptr(qkv), _row_major(qkv, "qkv"), B * T, T, H, Hkv, hd, _lib.ptr(q_w),
+                                       _lib.ptr(k_w), ctypes.c_float(eps), _lib.ptr(inv_freq), _lib.ptr(raw), _lib.ptr(rstd),
+                                       _lib.num_sms(), _lib.stream_ptr()), "qk_norm_rope_fwd")
+    _tick()
+    return qkv
+
+
+def qk_norm_rope_bwd(dqkv, B, T, H, Hkv, hd, q_w, k_w, inv_freq, raw, rstd, dq_w, dk_w):
+    """Backward of :func:`qk_norm_rope_fwd`, in place on the q|k part of ``dqkv``; the norm-weight gradients ``dq_w`` /
+    ``dk_w`` (fp32 [hd]) are accumulated."""
+    if not _qk_norm_kernel_ok(dqkv, hd):
+        return ref.qk_norm_rope_bwd(dqkv, B, T, H, Hkv, hd, q_w, k_w, inv_freq, raw, rstd, dq_w, dk_w)
+    _c(_lib.lib().dtb_qk_norm_rope_bwd(_lib.ptr(dqkv), _row_major(dqkv, "dqkv"), B * T, T, H, Hkv, hd, _lib.ptr(q_w),
+                                       _lib.ptr(k_w), _lib.ptr(inv_freq), _lib.ptr(raw), _lib.ptr(rstd), _lib.ptr(dq_w),
+                                       _lib.ptr(dk_w), _lib.num_sms(), _lib.stream_ptr()), "qk_norm_rope_bwd")
+    _tick()
+    return dqkv
+
+
 def ce_fwd_bwd(logits, targets, V, losses, grad_scale):
     if not use_kernels(logits):
         return ref.ce_fwd_bwd(logits, targets, V, losses, grad_scale)

@@ -293,6 +293,53 @@ def rope_(qkv, B, T, H, Hkv, hd, theta, inverse=False, inv_freq=None):
     return qkv
 
 
+def _qk_norm_weights(q_w, k_w, H, Hkv):
+    """[H + Hkv, hd] fp32: q_norm for the q heads, k_norm for the k heads."""
+    return torch.cat([q_w.float()[None].expand(H, -1), k_w.float()[None].expand(Hkv, -1)])
+
+
+def _rotate(x, T, inv, sign):  # x [B, T, h, hd] fp32, rotate-half by sign * t * inv
+    half = x.shape[-1] // 2
+    ang = torch.arange(T, device=x.device, dtype=torch.float32)[:, None] * inv.to(device=x.device, dtype=torch.float32)[None, :]
+    c, s = ang.cos()[None, :, None, :], sign * ang.sin()[None, :, None, :]
+    x1, x2 = x[..., :half], x[..., half:]
+    return torch.cat([x1 * c - x2 * s, x2 * c + x1 * s], dim=-1)
+
+
+def qk_norm_rope_fwd(qkv, B, T, H, Hkv, hd, q_w, k_w, eps, inv_freq, raw=None, rstd=None):
+    """In place on the q|k part of packed qkv [B*T, (H+2Hkv)*hd]: per-head RMSNorm (``q_w`` for q heads, ``k_w`` for k heads,
+    fp32 statistics) followed by rotate-half RoPE with the ``inv_freq`` table [hd/2].  v is not touched.  Optional saves
+    for the backward: ``raw`` [B*T, (H+Hkv)*hd] = the q|k input, ``rstd`` [B*T, H+Hkv] fp32."""
+    nh = H + Hkv
+    x = qkv.view(B, T, H + 2 * Hkv, hd)
+    qk = x[:, :, :nh].float()
+    if raw is not None:
+        raw.copy_(x[:, :, :nh].reshape(B * T, nh * hd))
+    rs = torch.rsqrt(qk.pow(2).mean(-1) + eps)
+    if rstd is not None:
+        rstd.copy_(rs.reshape(B * T, nh))
+    y = qk * rs[..., None] * _qk_norm_weights(q_w, k_w, H, Hkv)
+    x[:, :, :nh].copy_(_rotate(y, T, inv_freq, 1.0).to(qkv.dtype))
+    return qkv
+
+
+def qk_norm_rope_bwd(dqkv, B, T, H, Hkv, hd, q_w, k_w, inv_freq, raw, rstd, dq_w, dk_w):
+    """Backward of :func:`qk_norm_rope_fwd`, in place on the q|k part of dqkv: g = R(-theta) dy, x^ = raw * rstd,
+    dx = rstd * (g w - x^ mean(g w x^)); ``dq_w`` / ``dk_w`` (fp32 [hd]) += sum of g x^ over rows and q / k heads."""
+    nh = H + Hkv
+    d = dqkv.view(B, T, H + 2 * Hkv, hd)
+    g = _rotate(d[:, :, :nh].float(), T, inv_freq, -1.0)
+    rs = rstd.view(B, T, nh, 1).float()
+    xh = raw.view(B, T, nh, hd).float() * rs
+    gw = g * _qk_norm_weights(q_w, k_w, H, Hkv)
+    dx = rs * (gw - xh * (gw * xh).mean(-1, keepdim=True))
+    gx = g * xh
+    dq_w.add_(gx[:, :, :H].sum((0, 1, 2)).to(dq_w.dtype))
+    dk_w.add_(gx[:, :, H:].sum((0, 1, 2)).to(dk_w.dtype))
+    d[:, :, :nh].copy_(dx.to(dqkv.dtype))
+    return dqkv
+
+
 def swiglu_fwd(gu, out):
     """gu [M, 2F] = [gate | up] -> out [M,F] = silu(gate) * up."""
     Fdim = gu.shape[-1] // 2
